@@ -120,6 +120,11 @@ def _declare(lib):
         'hsk_rank_metrics': (i32, [vp, i32, i32, C.POINTER(C.c_int), i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]),
         'hsk_rank_metrics_dense': (i32, [vp, i32, i32, C.POINTER(C.c_int), i32, vp, vp, i64, vp, i32, vp, vp, vp, vp,
                                          vp]),
+        'hsk_det_scratch_bytes': (i64, [i32, i32, i32]),
+        'hsk_mf_scatter_grads_det': (i32, [T, T, vp, vp, vp, i32, i32, vp, i64, vp, vp]),
+        'hsk_mf_train_fused_det': (i32, [T, T, vp, vp, i32, i32, i32, f32, vp, vp, vp, vp, i64, vp, vp]),
+        'hsk_rec_loss_det': (i32, [vp, vp, i32, i32, i32, f32, f32, vp, vp, vp, vp, i64, vp]),
+        'hsk_rank_metrics_sums_det': (i32, [vp, i32, i32, vp, vp, i32, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -716,3 +721,58 @@ def rank_metrics_dense(top_ids, ks, u_idx, y_true, discount, sums, counts, user_
                                             y_true.data_ptr(), y_true.shape[1], _ptr(user_group), n_groups,
                                             discount.data_ptr(), _ptr(per_user), sums.data_ptr(), counts.data_ptr(), st),
                'hsk_rank_metrics_dense')
+
+
+# ---- deterministic mode (hsk_det.cu) ----
+def det_scratch_bytes(B: int, N1: int, ld: int) -> int:
+    return int(lib().hsk_det_scratch_bytes(B, N1, ld))
+
+
+def _scratch_bytes(scratch) -> int:
+    return scratch.numel() * scratch.element_size()
+
+
+def mf_scatter_grads_det(tables: MfTables, grads: MfTables, u_idx, i_idx, dscores, scratch, status=None):
+    """hsk_mf_scatter_grads_det: the touched rows of `grads` are STORED (fixed summation order, no atomics)."""
+    _req(u_idx, torch.int64, 'u_idx'); _req(i_idx, torch.int64, 'i_idx'); _req(dscores, torch.float32, 'dscores')
+    B, N1 = i_idx.shape
+    with _on_device_of(u_idx, i_idx, dscores, scratch, status) as st:
+        _check(lib().hsk_mf_scatter_grads_det(C.byref(tables), C.byref(grads), u_idx.data_ptr(), i_idx.data_ptr(),
+                                              dscores.data_ptr(), B, N1, scratch.data_ptr(), _scratch_bytes(scratch),
+                                              _ptr(status), st), 'hsk_mf_scatter_grads_det')
+
+
+def mf_train_fused_det(tables: MfTables, grads: MfTables, u_idx, i_idx, loss_kind: int, neg_shift: float, loss_accum,
+                       scratch, scores_out=None, dscores_out=None, status=None):
+    """hsk_mf_train_fused_det: the fused step with per-sample dL/ds and a fixed-order scatter / loss sum."""
+    _req(u_idx, torch.int64, 'u_idx'); _req(i_idx, torch.int64, 'i_idx'); _req(loss_accum, torch.float64, 'loss_accum')
+    B, N1 = i_idx.shape
+    with _on_device_of(u_idx, i_idx, loss_accum, scratch, scores_out, dscores_out, status) as st:
+        _check(lib().hsk_mf_train_fused_det(C.byref(tables), C.byref(grads), u_idx.data_ptr(), i_idx.data_ptr(), B, N1,
+                                            loss_kind, neg_shift, loss_accum.data_ptr(), _ptr(scores_out),
+                                            _ptr(dscores_out), scratch.data_ptr(), _scratch_bytes(scratch), _ptr(status),
+                                            st), 'hsk_mf_train_fused_det')
+
+
+def rec_loss_det(scores, labels, loss_kind: int, neg_shift: float, grad_scale: float, loss_accum, dscores, scratch,
+                 shifted_out=None):
+    """hsk_rec_loss_det: hsk_rec_loss with the per-row losses summed in a fixed order (scratch >= 8 * B bytes)."""
+    _req(scores, torch.float32, 'scores'); _req(loss_accum, torch.float64, 'loss_accum'); _req(dscores, torch.float32, 'dscores')
+    if labels is not None:
+        _req(labels, torch.float64, 'labels')
+    B, N1 = scores.shape
+    with _on_device_of(scores, labels, loss_accum, dscores, shifted_out, scratch) as st:
+        _check(lib().hsk_rec_loss_det(scores.data_ptr(), _ptr(labels), B, N1, loss_kind, neg_shift, grad_scale,
+                                      loss_accum.data_ptr(), dscores.data_ptr(), _ptr(shifted_out), scratch.data_ptr(),
+                                      _scratch_bytes(scratch), st), 'hsk_rec_loss_det')
+
+
+def rank_metrics_sums_det(per_user, u_idx, sums, user_group=None, n_groups=0):
+    """sums [(1 + n_groups), n_ks, 3] += fixed-order sums of per_user [Be, n_ks, 3] (hsk_rank_metrics_sums_det)."""
+    _req(per_user, torch.float32, 'per_user'); _req(u_idx, torch.int64, 'u_idx'); _req(sums, torch.float64, 'sums')
+    if user_group is not None:
+        _req(user_group, torch.int32, 'user_group')
+    Be, n_ks, _ = per_user.shape
+    with _on_device_of(per_user, u_idx, sums, user_group) as st:
+        _check(lib().hsk_rank_metrics_sums_det(per_user.data_ptr(), Be, n_ks, u_idx.data_ptr(), _ptr(user_group), n_groups,
+                                               sums.data_ptr(), st), 'hsk_rank_metrics_sums_det')

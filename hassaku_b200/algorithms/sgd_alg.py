@@ -15,7 +15,7 @@ from typing import Tuple, Union
 import torch
 from torch import nn
 
-from hassaku_b200 import _C
+from hassaku_b200 import _C, determinism
 from hassaku_b200.algorithms.base_classes import SGDBasedRecommenderAlgorithm
 from hassaku_b200.train.utils import general_weight_init
 
@@ -66,7 +66,8 @@ class ArenaLayout:
 
 class _MfScoreFn(torch.autograd.Function):
     """forward = hsk_mf_scores; backward = hsk_mf_scatter_grads into fresh dense gradient tables (what autograd +
-    aten::embedding_dense_backward do in the reference, SURVEY §2b K4)."""
+    aten::embedding_dense_backward do in the reference, SURVEY §2b K4); hsk_mf_scatter_grads_det under
+    torch.use_deterministic_algorithms(True)."""
 
     @staticmethod
     def forward(ctx, model, u_idxs, i_idxs, Uw, Vw, Ub, Ib, Gb):
@@ -82,8 +83,14 @@ class _MfScoreFn(torch.autograd.Function):
         u_idxs, i_idxs = ctx.saved_tensors
         lay = model.layout
         g_arena = torch.zeros(lay.n_total, dtype=torch.float32, device=dscores.device)
-        _C.mf_scatter_grads(model._tables(), lay.tables(g_arena), u_idxs, i_idxs,
-                            dscores.contiguous().float(), model._status())
+        if determinism.enabled():
+            scratch = determinism.scratch(model, _C.det_scratch_bytes(i_idxs.shape[0], i_idxs.shape[1], lay.ld),
+                                          dscores.device)
+            _C.mf_scatter_grads_det(model._tables(), lay.tables(g_arena), u_idxs, i_idxs, dscores.contiguous().float(),
+                                    scratch, model._status())
+        else:
+            _C.mf_scatter_grads(model._tables(), lay.tables(g_arena), u_idxs, i_idxs,
+                                dscores.contiguous().float(), model._status())
         grads = lay.views(g_arena)   # (gU, gV, gUb, gIb, gGb); None where the model has no such table
         need = ctx.needs_input_grad[3:]
         return (None, None, None) + tuple(g if n else None for g, n in zip(grads, need))

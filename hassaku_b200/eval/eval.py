@@ -15,7 +15,7 @@ import numpy as np
 import torch
 from tqdm import tqdm
 
-from hassaku_b200 import _C, nvtx
+from hassaku_b200 import _C, determinism, nvtx
 from hassaku_b200.algorithms.base_classes import RecommenderAlgorithm
 from hassaku_b200.algorithms.sgd_alg import SGDMatrixFactorization
 from hassaku_b200.eval.metrics import (dense_topk, discount_table, hellinger_distance, hit_from_precision,
@@ -104,6 +104,22 @@ class FullEvaluator:
             return None
         return torch.empty((B, len(self.K_VALUES), 3), dtype=torch.float32, device=device)
 
+    def _metric_outputs(self, B, device):
+        """(per_user buffer or None, the sums hsk_rank_metrics adds into).  Under torch.use_deterministic_algorithms the
+        kernel's atomic sums go to a discarded buffer and `_det_sums` adds the per-user rows in a fixed order."""
+        per_user = self._per_user_buf(B, device)
+        if not determinism.enabled():
+            return per_user, self._sums
+        if per_user is None:
+            per_user = torch.empty((B, len(self.K_VALUES), 3), dtype=torch.float32, device=device)
+        if getattr(self, '_discard', None) is None or self._discard.shape != self._sums.shape:
+            self._discard = torch.zeros_like(self._sums)
+        return per_user, self._discard
+
+    def _det_sums(self, u_idxs, per_user, sums):
+        if sums is not self._sums:
+            _C.rank_metrics_sums_det(per_user, u_idxs, self._sums, user_group=self._group_dev, n_groups=self.n_groups)
+
     def _keep(self, u_idxs, per_user):
         if per_user is None:
             return
@@ -124,9 +140,10 @@ class FullEvaluator:
         _, ids = dense_topk(logits, ks[0])  # eval.py:61-63
         u = u_idxs.to(dev, torch.int64).contiguous()
         y = y_true.to(dev, torch.float32).contiguous()
-        per_user = self._per_user_buf(len(u), dev)
-        _C.rank_metrics_dense(ids, ks, u, y, discount_table(ks[0], dev), self._sums, self._counts,
+        per_user, sums = self._metric_outputs(len(u), dev)
+        _C.rank_metrics_dense(ids, ks, u, y, discount_table(ks[0], dev), sums, self._counts,
                               user_group=self._group_dev, n_groups=self.n_groups, per_user=per_user)
+        self._det_sums(u, per_user, sums)
         self._keep(u, per_user)
 
     # ---- fused path: ranked ids + CSR labels ----
@@ -136,9 +153,10 @@ class FullEvaluator:
         self._prepare(dev)
         ks = self._ks()
         assert top_ids.shape[-1] == ks[0], 'Top-k indexes have different "k" compared to K_VALUES'
-        per_user = self._per_user_buf(len(u_idxs), dev)
-        _C.rank_metrics(top_ids, ks, u_idxs, labels.indptr, labels.indices, discount_table(ks[0], dev), self._sums,
+        per_user, sums = self._metric_outputs(len(u_idxs), dev)
+        _C.rank_metrics(top_ids, ks, u_idxs, labels.indptr, labels.indices, discount_table(ks[0], dev), sums,
                         self._counts, user_group=self._group_dev, n_groups=self.n_groups, per_user=per_user)
+        self._det_sums(u_idxs, per_user, sums)
         self._keep(u_idxs, per_user)
 
     def get_results(self):

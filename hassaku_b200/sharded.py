@@ -42,7 +42,7 @@ from typing import Dict, Optional
 import torch
 import torch.distributed as dist
 
-from hassaku_b200 import _C, nvtx
+from hassaku_b200 import _C, determinism, nvtx
 from hassaku_b200.algorithms.sgd_alg import ArenaLayout
 
 
@@ -541,7 +541,10 @@ class ShardedMF:
         self._peer = None
 
     def step(self, u_global, i_global, B_global, loss_kind, neg_shift, lr, wd, decoupled=True, exchange='auto', capq=None):
-        """Dispatch on the expected fraction of distinct items: dense exchange when the batch covers the item table."""
+        """Dispatch on the expected fraction of distinct items: dense exchange when the batch covers the item table.
+        Raises under torch.use_deterministic_algorithms(True) (warns under warn_only): the exchanges reduce gradients
+        from several ranks with floating-point atomics, and there is no deterministic implementation yet."""
+        determinism.alert_not_deterministic('ShardedMF.step')
         if exchange in ('auto', 'auto_graph'):
             dense = i_global.numel() >= 2 * self.spec.n_items // self.spec.world
             exchange = ('dense' if dense else 'sparse') + ('_graph' if exchange == 'auto_graph' else '')

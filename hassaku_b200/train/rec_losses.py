@@ -10,7 +10,7 @@ from enum import Enum
 
 import torch
 
-from hassaku_b200 import _C
+from hassaku_b200 import _C, determinism
 
 
 class RecommenderSystemLoss(ABC):
@@ -55,7 +55,11 @@ class _RecLossFn(torch.autograd.Function):
             lab = labels.detach().to(x.device, torch.float64).contiguous()
         loss = torch.zeros(1, dtype=torch.float64, device=x.device)
         ds = torch.empty_like(x)
-        _C.rec_loss(x, lab, kind, shift, 1.0, loss, ds, x if mutate else None)
+        if determinism.enabled():   # fixed-order sum of the per-row losses
+            scratch = torch.empty(8 * x.shape[0], dtype=torch.uint8, device=x.device)
+            _C.rec_loss_det(x, lab, kind, shift, 1.0, loss, ds, scratch, x if mutate else None)
+        else:
+            _C.rec_loss(x, lab, kind, shift, 1.0, loss, ds, x if mutate else None)
         # (the in-place shift goes through the detached alias: nothing upstream saved the model output)
         ctx.save_for_backward(ds)
         return loss[0].to(out_dtype)

@@ -1,7 +1,7 @@
 """One fused training step of SGDMatrixFactorization (train/trainer.py:133-148 of the reference)."""
 import torch
 
-from hassaku_b200 import _C, nvtx
+from hassaku_b200 import _C, determinism, nvtx
 from hassaku_b200.train.optim import DenseAdam
 from hassaku_b200.train.rec_losses import RecommenderSystemLoss
 
@@ -55,8 +55,15 @@ class FusedMFTrainStep:
             i = i_idxs.to(self.device, torch.int64).contiguous()
         else:
             slot, u, i = self._stage(u_idxs, i_idxs)
-        _C.mf_train_fused(self.model._tables(), self.optimizer.grad_tables, u, i, self.kind, self.shift,
-                          self.loss_accum if loss_out is None else loss_out, status=self.model._status())
+        loss = self.loss_accum if loss_out is None else loss_out
+        if determinism.enabled():
+            scratch = determinism.scratch(self, _C.det_scratch_bytes(i.shape[0], i.shape[1], self.model.layout.ld),
+                                          self.device)
+            _C.mf_train_fused_det(self.model._tables(), self.optimizer.grad_tables, u, i, self.kind, self.shift, loss,
+                                  scratch, status=self.model._status())
+        else:
+            _C.mf_train_fused(self.model._tables(), self.optimizer.grad_tables, u, i, self.kind, self.shift, loss,
+                              status=self.model._status())
         if hasattr(self.optimizer, 'mark'):
             self.optimizer.mark(u, i)
         self.optimizer.step_fused()

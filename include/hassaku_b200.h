@@ -396,6 +396,41 @@ HSK_API int hsk_adamw_consts(double lr, double beta1, double beta2, double eps, 
 HSK_API int hsk_adamw_dense_graph(float* p, float* m, float* v, float* g, int64_t n, const float* consts_dev,
                                   int decoupled_decay, int adam_l2, int zero_grad, hsk_stream_t stream);
 
+/* ==== deterministic mode (hsk_det.cu): bitwise-reproducible training / evaluation reductions ========================
+ * What the Python layer runs under torch.use_deterministic_algorithms(True).  The batch is grouped by row (stable radix
+ * sort of the item ids of the B * N1 slots and of the user ids of the B samples) and every touched row is produced by ONE
+ * warp as a fixed-order sum: no floating-point atomics, the same bits on every run, grid and GPU.
+ * Order (restated bit for bit by oracle/det_oracle.py): slot s = b * N1 + j; a row's entries are taken in increasing s;
+ * they are cut into chunks at the row's ends and at every multiple of C = 32 of the entry's position in the sorted list
+ * (the user list expands every sample into its N1 slots); within a chunk acc = +0, acc = fadd_rn(acc, fmul_rn(ds_s,
+ * other_row)) (other_row = Uw[u_b] for an item row, Vw[i_s] for a user row; bias: acc_b = fadd_rn(acc_b, ds_s)); the
+ * row is the chunk partials added in order from the first.  gGb: chunks of 1024 consecutive slots, the same way.
+ * Unlike hsk_mf_scatter_grads the rows are STORED: every row the batch touches is overwritten with its gradient (g must
+ * be zero there to get the same result as the accumulating kernels); rows it does not touch are not written.
+ * Scratch: device memory of hsk_det_scratch_bytes(B, N1, ld) bytes, 16-byte aligned, owned by the caller.
+ *   hsk_mf_scatter_grads_det   = hsk_mf_scatter_grads with the order above.  An entry whose user / item is out of range is
+ *       skipped and reported in status.
+ *   hsk_mf_train_fused_det     = hsk_mf_train_fused: per sample the fused kernels' scores, loss term and dL/ds (a sample
+ *       with an out-of-range index is skipped: dL/ds 0, loss 0), then the scatter above; *loss_accum += the per-sample
+ *       fp64 losses summed in a fixed order.  N1 <= 10240.
+ *   hsk_rec_loss_det           = hsk_rec_loss (dscores required, not aliasing scores) with the per-row losses summed in a
+ *       fixed order; scratch >= 8 * B bytes.
+ *   hsk_rank_metrics_sums_det  sums[g] += the fixed-order sum of per_user [Be, n_ks, 3] (hsk_rank_metrics' per-user
+ *       output) over the batch's users of group g - 1 (g = 0: all users), g < 1 + n_groups: the deterministic
+ *       replacement of hsk_rank_metrics' floating-point sums (its integer counts are exact as they are). */
+HSK_API int64_t hsk_det_scratch_bytes(int B, int N1, int ld);
+HSK_API int hsk_mf_scatter_grads_det(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx,
+                                     const float* dscores, int B, int N1, void* scratch, int64_t scratch_bytes, int32_t* status,
+                                     hsk_stream_t stream);
+HSK_API int hsk_mf_train_fused_det(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx,
+                                   int B, int N1, int loss_kind, float neg_shift, double* loss_accum, float* scores_out,
+                                   float* dscores_out, void* scratch, int64_t scratch_bytes, int32_t* status, hsk_stream_t stream);
+HSK_API int hsk_rec_loss_det(const float* scores, const double* labels, int B, int N1, int loss_kind, float neg_shift,
+                             float grad_scale, double* loss_accum, float* dscores, float* shifted_out /* nullable */,
+                             void* scratch, int64_t scratch_bytes, hsk_stream_t stream);
+HSK_API int hsk_rank_metrics_sums_det(const float* per_user, int Be, int n_ks, const int64_t* u_idx,
+                                      const int32_t* user_group /* nullable */, int n_groups, double* sums, hsk_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
