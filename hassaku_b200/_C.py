@@ -125,6 +125,9 @@ def _declare(lib):
         'hsk_mf_train_fused_det': (i32, [T, T, vp, vp, i32, i32, i32, f32, vp, vp, vp, vp, i64, vp, vp]),
         'hsk_rec_loss_det': (i32, [vp, vp, i32, i32, i32, f32, f32, vp, vp, vp, vp, i64, vp]),
         'hsk_rank_metrics_sums_det': (i32, [vp, i32, i32, vp, vp, i32, vp, vp]),
+        'hsk_mf_train_fused_pack': (i32, [T, T, i64, i32, vp, i32, vp, vp, i32, i32, i32, f32, vp, vp, vp]),
+        'hsk_adamw_pack': (i32, [vp, vp, vp, vp, i64, i32, vp, i32, vp, C.POINTER(RowSegment), i32, i64, i32, vp, vp]),
+        'hsk_adamw_consts_table': (i32, [vp, vp, i32, f64, f64, f64, i64, i32, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -443,19 +446,82 @@ def adamw_dense_rows(p, m, v, g, segments, lr, beta1, beta2, eps, weight_decay, 
     gradient traffic is skipped for rows not stamped this step; everything else takes the plain dense path."""
     for n, t in (('p', p), ('m', m), ('v', v), ('g', g)):
         _req(t, torch.float32, n)
-    segs = list(segments)
-    arr = (RowSegment * max(len(segs), 1))()
-    for k, (off, rows, ld, stamps) in enumerate(segs):
-        _req(stamps, torch.uint8, 'stamps')
-        if stamps.numel() < rows:
-            raise HskError('adamw_dense_rows: stamp array shorter than the segment')
-        arr[k] = RowSegment(off, rows, ld, stamps.data_ptr())
+    segs, arr = _row_segments(segments, 'adamw_dense_rows')
     if consts_dev is not None:
         _req(consts_dev, torch.float32, 'consts_dev'); _req(step_dev, torch.int64, 'step_dev')
     with _on_device_of(p, m, v, g, consts_dev, step_dev, *[sg[3] for sg in segs]) as st:
         _check(lib().hsk_adamw_dense_rows(p.data_ptr(), m.data_ptr(), v.data_ptr(), g.data_ptr(), p.numel(), arr, len(segs),
                                           lr, beta1, beta2, eps, weight_decay, step, _ptr(consts_dev), _ptr(step_dev), arith,
                                           int(adam_l2), st), 'hsk_adamw_dense_rows')
+
+
+def _row_segments(segments, who):
+    segs = list(segments)
+    arr = (RowSegment * max(len(segs), 1))()
+    for k, (off, rows, ld, stamps) in enumerate(segs):
+        _req(stamps, torch.uint8, 'stamps')
+        if stamps.numel() < rows:
+            raise HskError(f'{who}: stamp array shorter than the segment')
+        arr[k] = RowSegment(off, rows, ld, stamps.data_ptr())
+    return segs, arr
+
+
+# ---- trial pack: M models of one shape, [M, stride] arenas ----
+def _pack_rows(name, t, n_trials: int):
+    """t: [n_trials, stride] fp32 CUDA, rows contiguous -> stride."""
+    _req(t, torch.float32, name)
+    if t.dim() != 2 or t.shape[0] != n_trials:
+        raise HskError(f'{name} must be [n_trials, stride] with n_trials = {n_trials}')
+    return t.shape[1]
+
+
+def mf_train_fused_pack(tables: MfTables, grads: MfTables, trial_stride: int, n_trials: int, active, u_idx, i_idx,
+                        loss_kind: int, neg_shift: float, loss_accum, status=None):
+    """hsk_mf_train_fused_pack: the fused step of every trial listed in `active` (int32 device) on one shared batch;
+    tables / grads = trial 0's, trial j's at + j * trial_stride elements; loss_accum fp64 [n_trials]."""
+    _req(u_idx, torch.int64, 'u_idx'); _req(i_idx, torch.int64, 'i_idx'); _req(active, torch.int32, 'active')
+    _req(loss_accum, torch.float64, 'loss_accum')
+    if loss_accum.numel() != n_trials:
+        raise HskError(f'loss_accum must hold n_trials = {n_trials} accumulators')
+    B, N1 = i_idx.shape
+    with _on_device_of(u_idx, i_idx, active, loss_accum, status) as st:
+        _check(lib().hsk_mf_train_fused_pack(C.byref(tables), C.byref(grads), trial_stride, n_trials, active.data_ptr(),
+                                             active.numel(), u_idx.data_ptr(), i_idx.data_ptr(), B, N1, loss_kind, neg_shift,
+                                             loss_accum.data_ptr(), _ptr(status), st), 'hsk_mf_train_fused_pack')
+
+
+def adamw_pack(p, m, v, g, active, consts_dev, segments=(), step: int = 0, adam_l2: bool = False, status=None):
+    """hsk_adamw_pack over [n_trials, stride] arenas: consts_dev fp32 [n_trials, 8] (this step's hsk_adamw_consts per
+    trial); segments (offset inside one trial's row, n_rows, ld, stamps) select the row-stamped form."""
+    n_trials = p.shape[0]
+    stride = _pack_rows('p', p, n_trials)
+    for n, t in (('m', m), ('v', v), ('g', g)):
+        if _pack_rows(n, t, n_trials) != stride:
+            raise HskError('adamw_pack: p, m, v, g must have one shape')
+    _req(active, torch.int32, 'active'); _req(consts_dev, torch.float32, 'consts_dev')
+    if consts_dev.numel() != 8 * n_trials:
+        raise HskError(f'consts_dev must be [n_trials, 8] = [{n_trials}, 8]')
+    segs, arr = _row_segments(segments, 'adamw_pack')
+    with _on_device_of(p, m, v, g, active, consts_dev, status, *[sg[3] for sg in segs]) as st:
+        _check(lib().hsk_adamw_pack(p.data_ptr(), m.data_ptr(), v.data_ptr(), g.data_ptr(), stride, n_trials, active.data_ptr(),
+                                    active.numel(), consts_dev.data_ptr(), arr, len(segs), step, int(adam_l2), _ptr(status), st),
+               'hsk_adamw_pack')
+
+
+def adamw_consts_table(lrs, wds, beta1: float, beta2: float, eps: float, first_step: int, n_steps: int, out_host=None):
+    """Host fp32 [n_steps, n_trials, 8]: hsk_adamw_consts of trial j at step first_step + s (hsk_adamw_consts_table)."""
+    M = len(lrs)
+    if len(wds) != M:
+        raise HskError('adamw_consts_table: one weight decay per learning rate')
+    if out_host is None:
+        out_host = torch.empty((n_steps, M, 8), dtype=torch.float32)
+    if out_host.is_cuda or out_host.dtype != torch.float32 or out_host.numel() < n_steps * M * 8 or not out_host.is_contiguous():
+        raise HskError('adamw_consts_table: out_host must be a contiguous host fp32 tensor of n_steps * n_trials * 8')
+    lr_a = (C.c_double * M)(*[float(x) for x in lrs])
+    wd_a = (C.c_double * M)(*[float(x) for x in wds])
+    _check(lib().hsk_adamw_consts_table(lr_a, wd_a, M, beta1, beta2, eps, first_step, n_steps, out_host.data_ptr()),
+           'hsk_adamw_consts_table')
+    return out_host
 
 
 def adagrad_dense(p, state_sum, g, lr, eps=1e-10, weight_decay=0.0, zero_grad=True):

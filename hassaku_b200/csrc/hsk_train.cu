@@ -179,195 +179,14 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) mf_scatter_kernel(TrainArgs
 // ------------------------------------------------------------------------------------------------
 template <int NV, int LOSS>
 __global__ void __launch_bounds__(kWarpsPerCta * 32) mf_train_fused_kernel(TrainArgs a) {
-    extern __shared__ float sm_scores[];  // [N1] (sampled-softmax only)
-    __shared__ float4 sm_gu[kWarpsPerCta][NV][32];
-    __shared__ float sm_ds0[kWarpsPerCta];
-    __shared__ float sm_dsum[kWarpsPerCta];
-    __shared__ double sm_loss[kWarpsPerCta];
-    __shared__ float sm_lse;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int b = blockIdx.x;
-    const int64_t u = a.u_idx[b];
-    const int64_t* irow = a.i_idx + (int64_t)b * a.N1;
-    const int64_t i0 = irow[0];
-    if (bad_index(u, a.n_users) || bad_index(i0, a.n_items)) {
-        if (threadIdx.x == 0 && a.status) atomicOr(a.status, HSK_STATUS_BAD_INDEX);
-        return;
-    }
-    Row<NV> ur, gu;
-    ur.load(a.Uw + u * a.ld, a.nvec, lane);
-    gu.zero();
-    const float bias_u = a.Ub ? a.Ub[u] : 0.f;
-    const float gb = a.Gb ? a.Gb[0] : 0.f;
-    auto finish_score = [&](float dotv, int64_t it) {
-        float s = dotv;
-        if (a.Ub) s += bias_u;
-        if (a.Ib) s += a.Ib[it];
-        if (a.Gb) s += gb;
-        return s;
-    };
-    float ds0 = 0.f;    // dL/ds of the positive slot accumulated by this warp (bpr) / whole value (others, warp 0)
-    float dsum = 0.f;   // sum of every dL/ds this warp produced (user / global bias gradients)
-    double loss_local = 0.0;
-    const int64_t rowoff = (int64_t)b * a.N1;
+#include "hsk_train_fused_body.inc"
+}
 
-    if (LOSS == HSK_LOSS_BPR) {
-        // positive row first (every warp: the other three hit L1), then one pass over this warp's negatives
-        Row<NV> v0;
-        v0.load(a.Vw + i0 * a.ld, a.nvec, lane);
-        const float s0 = finish_score(warp_sum(ur.dot_partial(v0)), i0);
-        const double inv = a.inv_count;
-        const int j0 = 1 + blockIdx.y * a.j_per_cta, j1 = min(a.N1, j0 + a.j_per_cta);
-        for (int j = j0 + warp; j < j1; j += kWarpsPerCta) {
-            const int64_t it = irow[j];
-            if (bad_index(it, a.n_items)) {
-                if (lane == 0 && a.status) atomicOr(a.status, HSK_STATUS_BAD_INDEX);
-                continue;
-            }
-            Row<NV> vr;
-            vr.load(a.Vw + it * a.ld, a.nvec, lane);
-            const float sj = finish_score(warp_sum(ur.dot_partial(vr)), it);
-            const float x = s0 - sj;
-            const float dx = (float)(((double)sigmoid_f(x) - 1.0) * inv);  // dL/dx
-            const float dsj = -dx;
-            ds0 += dx;
-            dsum += dsj;
-            gu.axpy(dsj, vr);
-            ur.red_scaled(a.gV + it * a.ld, dsj, a.nvec, lane);
-            if (lane == 0) {
-                loss_local += -(double)log_sigmoid_f(x) * inv;
-                if (a.gIb) atomicAdd(a.gIb + it, dsj);
-                if (a.scores_out) a.scores_out[rowoff + j] = sj;
-                if (a.dscores_out) a.dscores_out[rowoff + j] = dsj;
-            }
-        }
-        // combine the warps' partial user-row gradient and positive-slot gradient
-#pragma unroll
-        for (int k = 0; k < NV; ++k) sm_gu[warp][k][lane] = gu.v[k];
-        if (lane == 0) { sm_ds0[warp] = ds0; sm_dsum[warp] = dsum; sm_loss[warp] = loss_local; }
-        __syncthreads();
-        if (warp == 0) {
-            float d0 = 0.f, dsm = 0.f;
-            double ls = 0.0;
-#pragma unroll
-            for (int w = 0; w < kWarpsPerCta; ++w) { d0 += sm_ds0[w]; dsm += sm_dsum[w]; ls += sm_loss[w]; }
-#pragma unroll
-            for (int w = 1; w < kWarpsPerCta; ++w) {
-#pragma unroll
-                for (int k = 0; k < NV; ++k) {
-                    float4 o = sm_gu[w][k][lane];
-                    gu.v[k].x += o.x; gu.v[k].y += o.y; gu.v[k].z += o.z; gu.v[k].w += o.w;
-                }
-            }
-            gu.axpy(d0, v0);
-            gu.red(a.gU + u * a.ld, a.nvec, lane);
-            ur.red_scaled(a.gV + i0 * a.ld, d0, a.nvec, lane);
-            if (lane == 0) {
-                if (a.gIb) atomicAdd(a.gIb + i0, d0);
-                dsm += d0;
-                if (a.gUb) atomicAdd(a.gUb + u, dsm);
-                if (a.gGb) atomicAdd(a.gGb, dsm);
-                if (a.loss_accum && ls != 0.0) atomicAdd(a.loss_accum, ls);
-                if (blockIdx.y == 0 && a.scores_out) a.scores_out[rowoff] = s0;
-                // the positive slot's dL/ds is the sum over all gridDim.y CTAs of this sample
-                if (a.dscores_out) { if (gridDim.y == 1) a.dscores_out[rowoff] = d0; else atomicAdd(a.dscores_out + rowoff, d0); }
-            }
-        }
-        return;
-    }
-
-    if (LOSS == HSK_LOSS_BCE) {
-        const double inv = a.inv_count;
-        const int j0 = blockIdx.y * a.j_per_cta, j1 = min(a.N1, j0 + a.j_per_cta);
-        for (int j = j0 + warp; j < j1; j += kWarpsPerCta) {
-            const int64_t it = irow[j];
-            if (bad_index(it, a.n_items)) {
-                if (lane == 0 && a.status) atomicOr(a.status, HSK_STATUS_BAD_INDEX);
-                continue;
-            }
-            Row<NV> vr;
-            vr.load(a.Vw + it * a.ld, a.nvec, lane);
-            const float sj = finish_score(warp_sum(ur.dot_partial(vr)), it);
-            const double y = (j == 0) ? 1.0 : 0.0;
-            const float dsj = (float)(((double)sigmoid_f(sj) - y) * inv);
-            dsum += dsj;
-            gu.axpy(dsj, vr);
-            ur.red_scaled(a.gV + it * a.ld, dsj, a.nvec, lane);
-            if (lane == 0) {
-                loss_local += ((1.0 - y) * (double)sj - (double)log_sigmoid_f(sj)) * inv;
-                if (a.gIb) atomicAdd(a.gIb + it, dsj);
-                if (a.scores_out) a.scores_out[rowoff + j] = sj;
-                if (a.dscores_out) a.dscores_out[rowoff + j] = dsj;
-            }
-        }
-    } else {  // sampled softmax: pass 1 scores -> smem, block-wide logsumexp, pass 2 gradients (rows re-read from L1/L2)
-        for (int j = warp; j < a.N1; j += kWarpsPerCta) {
-            const int64_t it = irow[j];
-            float sj = -INFINITY;
-            if (!bad_index(it, a.n_items)) {
-                Row<NV> vr;
-                vr.load(a.Vw + it * a.ld, a.nvec, lane);
-                sj = finish_score(warp_sum(ur.dot_partial(vr)), it);
-                if (lane == 0 && a.scores_out) a.scores_out[rowoff + j] = sj;
-                sj += (j > 0 ? a.neg_shift : 0.f);
-            } else if (lane == 0 && a.status) {
-                atomicOr(a.status, HSK_STATUS_BAD_INDEX);
-            }
-            if (lane == 0) sm_scores[j] = sj;
-        }
-        __syncthreads();
-        if (warp == 0) {
-            float mx = -INFINITY;
-            for (int j = lane; j < a.N1; j += 32) mx = fmaxf(mx, sm_scores[j]);
-            mx = warp_max(mx);
-            float se = 0.f;
-            for (int j = lane; j < a.N1; j += 32) se += expf(sm_scores[j] - mx);
-            se = warp_sum(se);
-            if (lane == 0) sm_lse = mx + logf(se);
-        }
-        __syncthreads();
-        const float lse = sm_lse;
-        if (threadIdx.x == 0) loss_local += (double)(lse - sm_scores[0]) * a.inv_count;
-        for (int j = warp; j < a.N1; j += kWarpsPerCta) {
-            const int64_t it = irow[j];
-            if (bad_index(it, a.n_items)) continue;
-            const float dsj = (expf(sm_scores[j] - lse) - (j == 0 ? 1.f : 0.f)) * (float)a.inv_count;
-            Row<NV> vr;
-            vr.load(a.Vw + it * a.ld, a.nvec, lane);
-            dsum += dsj;
-            gu.axpy(dsj, vr);
-            ur.red_scaled(a.gV + it * a.ld, dsj, a.nvec, lane);
-            if (lane == 0) {
-                if (a.gIb) atomicAdd(a.gIb + it, dsj);
-                if (a.dscores_out) a.dscores_out[rowoff + j] = dsj;
-            }
-        }
-    }
-    // bce / sampled-softmax epilogue
-#pragma unroll
-    for (int k = 0; k < NV; ++k) sm_gu[warp][k][lane] = gu.v[k];
-    if (lane == 0) { sm_dsum[warp] = dsum; sm_loss[warp] = loss_local; }
-    __syncthreads();
-    if (warp == 0) {
-        float dsm = 0.f;
-        double ls = 0.0;
-#pragma unroll
-        for (int w = 0; w < kWarpsPerCta; ++w) { dsm += sm_dsum[w]; ls += sm_loss[w]; }
-#pragma unroll
-        for (int w = 1; w < kWarpsPerCta; ++w) {
-#pragma unroll
-            for (int k = 0; k < NV; ++k) {
-                float4 o = sm_gu[w][k][lane];
-                gu.v[k].x += o.x; gu.v[k].y += o.y; gu.v[k].z += o.z; gu.v[k].w += o.w;
-            }
-        }
-        gu.red(a.gU + u * a.ld, a.nvec, lane);
-        if (lane == 0) {
-            if (a.gUb) atomicAdd(a.gUb + u, dsm);
-            if (a.gGb) atomicAdd(a.gGb, dsm);
-            if (a.loss_accum && ls != 0.0) atomicAdd(a.loss_accum, ls);
-        }
-    }
+// trial pack (hsk_mf_train_fused_pack): gridDim.z walks the active trials, gridDim.x / y as the single-model kernel
+template <int NV, int LOSS>
+__global__ void __launch_bounds__(kWarpsPerCta * 32) mf_train_fused_pack_kernel(TrainArgs a, PackArgs pk) {
+    if (!pack_select_trial(a, pk)) return;
+#include "hsk_train_fused_body.inc"
 }
 
 // ---- host-side argument validation shared by the entry points ----
@@ -576,6 +395,64 @@ extern "C" int hsk_mf_train_fused_v(const hsk_mf_tables* t, const hsk_mf_tables*
         HSK_DISPATCH_NV(nv, (mf_train_fused_kernel<NV, HSK_LOSS_SAMPLED_SOFTMAX><<<grid, threads, smem, s>>>(a)));
     }
     return check_launch("hsk_mf_train_fused");
+}
+
+extern "C" int hsk_mf_train_fused_pack(const hsk_mf_tables* t, const hsk_mf_tables* g, int64_t trial_stride, int n_trials,
+                                       const int32_t* active, int n_active, const int64_t* u_idx, const int64_t* i_idx, int B,
+                                       int N1, int loss_kind, float neg_shift, double* loss_accum, int32_t* status,
+                                       hsk_stream_t stream) {
+    TrainArgs a;
+    HSK_REQUIRE(g, "hsk_mf_train_fused_pack: gradient tables are null");
+    int rc = fill_args(a, t, g, u_idx, i_idx, B, N1, "hsk_mf_train_fused_pack");
+    if (rc) return rc;
+    HSK_REQUIRE(loss_kind >= 0 && loss_kind <= 2, "hsk_mf_train_fused_pack: unknown loss kind %d", loss_kind);
+    HSK_REQUIRE(loss_kind != HSK_LOSS_BPR || N1 >= 2, "hsk_mf_train_fused_pack: bpr needs at least one negative");
+    HSK_REQUIRE(n_trials >= 1 && n_active >= 0 && n_active <= n_trials && n_active <= 65535,
+                "hsk_mf_train_fused_pack: need 0 <= n_active <= n_trials, n_trials >= 1, n_active <= 65535 (n_trials=%d n_active=%d)",
+                n_trials, n_active);
+    HSK_REQUIRE(n_active == 0 || active, "hsk_mf_train_fused_pack: active is null");
+    HSK_REQUIRE(trial_stride > 0 && trial_stride % 4 == 0,
+                "hsk_mf_train_fused_pack: trial_stride must be a positive multiple of 4 (%lld)", (long long)trial_stride);
+    if (B == 0 || n_active == 0) return HSK_OK;
+    a.status = status;
+    a.loss_kind = loss_kind;
+    a.neg_shift = neg_shift;
+    a.loss_accum = loss_accum;
+    a.inv_count = loss_kind == HSK_LOSS_BPR ? 1.0 / ((double)B * (double)(N1 - 1))
+                : loss_kind == HSK_LOSS_BCE ? 1.0 / ((double)B * (double)N1) : 1.0 / (double)B;
+    PackArgs pk;
+    pk.stride = trial_stride;
+    pk.active = active;
+    pk.n_trials = n_trials;
+    cudaStream_t s = as_stream(stream);
+    // HSK_TRAIN_AUTO's rules applied to the work of the whole launch (n_active * B samples); where AUTO would take the
+    // bulk-copy ring, the register-gather kernel runs instead (the ring is not packed)
+    const int64_t work = (int64_t)n_active * B;
+    if (train_fused_q_fits(work, a.nvec, N1, loss_kind, false)) {
+        a.j_per_cta = N1;
+        return launch_train_fused_q_pack(a, pk, n_active, loss_kind, s);
+    }
+    const int work_i = work < 0x7FFFFFFF ? (int)work : 0x7FFFFFFF;
+    const int nv = (a.nvec + 31) / 32;
+    const int threads = kWarpsPerCta * 32;
+    if (loss_kind == HSK_LOSS_BPR) {
+        a.j_per_cta = pick_j_per_cta(work_i, N1 - 1, true);
+        if (a.j_per_cta > 128) a.j_per_cta = 128;
+        dim3 grid(B, (N1 - 1 + a.j_per_cta - 1) / a.j_per_cta, n_active);
+        HSK_DISPATCH_NV(nv, (mf_train_fused_pack_kernel<NV, HSK_LOSS_BPR><<<grid, threads, 0, s>>>(a, pk)));
+    } else if (loss_kind == HSK_LOSS_BCE) {
+        a.j_per_cta = pick_j_per_cta(work_i, N1, true);
+        if (a.j_per_cta > 128) a.j_per_cta = 128;
+        dim3 grid(B, (N1 + a.j_per_cta - 1) / a.j_per_cta, n_active);
+        HSK_DISPATCH_NV(nv, (mf_train_fused_pack_kernel<NV, HSK_LOSS_BCE><<<grid, threads, 0, s>>>(a, pk)));
+    } else {
+        a.j_per_cta = N1;
+        dim3 grid(B, 1, n_active);
+        const size_t smem = sizeof(float) * (size_t)N1;
+        HSK_REQUIRE(smem <= 40 * 1024, "hsk_mf_train_fused_pack: sampled-softmax supports at most 10240 slots per sample");
+        HSK_DISPATCH_NV(nv, (mf_train_fused_pack_kernel<NV, HSK_LOSS_SAMPLED_SOFTMAX><<<grid, threads, smem, s>>>(a, pk)));
+    }
+    return check_launch("hsk_mf_train_fused_pack");
 }
 
 // ---- row gather / scatter-add used by the item-sharded step (hassaku_b200/sharded.py): the rows a peer asked for are

@@ -351,6 +351,34 @@ __global__ void __launch_bounds__(kQWarps * 32) mf_train_fused_peer_kernel(Train
     mf_train_fused_q_body<K4, LOSS, true>(a, pv);
 }
 
+template <int K4, int LOSS>
+__global__ void __launch_bounds__(kQWarps * 32) mf_train_fused_q_pack_kernel(TrainArgs a, PackArgs pk) {
+    if (!pack_select_trial(a, pk)) return;
+    PeerArgs none;     // never read: every use is behind `if (PEER)`
+    mf_train_fused_q_body<K4, LOSS, false>(a, none);
+}
+
+template <int LOSS>
+static int launch_q_pack(const TrainArgs& a, const PackArgs& pk, int n_active, cudaStream_t s) {
+    const int k4 = (a.nvec + 7) / 8;
+    const int spc = kQWarps * 4;
+    const dim3 grid((a.B + spc - 1) / spc, 1, n_active);
+    const size_t smem = (LOSS == HSK_LOSS_SAMPLED_SOFTMAX) ? sizeof(float) * (size_t)spc * a.N1 : 0;
+    switch (k4) {
+        case 1: mf_train_fused_q_pack_kernel<1, LOSS><<<grid, kQWarps * 32, smem, s>>>(a, pk); break;
+        case 2: mf_train_fused_q_pack_kernel<2, LOSS><<<grid, kQWarps * 32, smem, s>>>(a, pk); break;
+        case 3: mf_train_fused_q_pack_kernel<3, LOSS><<<grid, kQWarps * 32, smem, s>>>(a, pk); break;
+        default: mf_train_fused_q_pack_kernel<4, LOSS><<<grid, kQWarps * 32, smem, s>>>(a, pk); break;
+    }
+    return check_launch("hsk_mf_train_fused_pack(quarter-warp)");
+}
+
+int launch_train_fused_q_pack(const TrainArgs& a, const PackArgs& pk, int n_active, int loss_kind, cudaStream_t s) {
+    if (loss_kind == HSK_LOSS_BPR) return launch_q_pack<HSK_LOSS_BPR>(a, pk, n_active, s);
+    if (loss_kind == HSK_LOSS_BCE) return launch_q_pack<HSK_LOSS_BCE>(a, pk, n_active, s);
+    return launch_q_pack<HSK_LOSS_SAMPLED_SOFTMAX>(a, pk, n_active, s);
+}
+
 template <int LOSS>
 static int launch_q_peer(const TrainArgs& a, const PeerArgs& pv, cudaStream_t s) {
     const int k4 = (a.nvec + 7) / 8;
@@ -401,17 +429,21 @@ static int launch_q(const TrainArgs& a, cudaStream_t s) {
 // returns 1 (no launch) when the shape is not one this kernel is meant for: rows longer than 128 floats, batches too
 // small to fill the GPU with one quarter-warp per sample, softmax samples whose score strip does not fit, or shapes
 // where the warp-per-row ring measured faster
-int launch_train_fused_q(const TrainArgs& a, int loss_kind, cudaStream_t s) {
-    if (a.nvec > 32) return 1;
-    if (!a.force_q) {
-        if (a.B < 2048) return 1;
+bool train_fused_q_fits(int64_t n_samples, int nvec, int N1, int loss_kind, bool force) {
+    if (nvec > 32) return false;
+    if (!force) {
+        if (n_samples < 2048) return false;
         // measured on B200 (B 8192, N 100, tables in L2; scripts/kbench.py trainraw): at d = 128 bpr / bce are bound by L2
         // traffic (reads + REDs) in every layout and the bulk-copy ring is ~10 % ahead (160 vs 176 us); at d = 64 this
         // kernel is 1.9x faster (84 vs 162 us, the ring is bound by its per-row instruction count); sampled softmax
         // (two passes over the rows) is faster here at every d <= 128 (143 vs 165 us at d = 128)
-        if (loss_kind != HSK_LOSS_SAMPLED_SOFTMAX && a.nvec > 24) return 1;
+        if (loss_kind != HSK_LOSS_SAMPLED_SOFTMAX && nvec > 24) return false;
     }
-    if (loss_kind == HSK_LOSS_SAMPLED_SOFTMAX && (size_t)a.N1 * kQWarps * 4 * sizeof(float) > 40 * 1024) return 1;
+    return !(loss_kind == HSK_LOSS_SAMPLED_SOFTMAX && (size_t)N1 * kQWarps * 4 * sizeof(float) > 40 * 1024);
+}
+
+int launch_train_fused_q(const TrainArgs& a, int loss_kind, cudaStream_t s) {
+    if (!train_fused_q_fits(a.B, a.nvec, a.N1, loss_kind, a.force_q != 0)) return 1;
     if (loss_kind == HSK_LOSS_BPR) return launch_q<HSK_LOSS_BPR>(a, s);
     if (loss_kind == HSK_LOSS_BCE) return launch_q<HSK_LOSS_BCE>(a, s);
     return launch_q<HSK_LOSS_SAMPLED_SOFTMAX>(a, s);

@@ -9,6 +9,20 @@ import torch
 from hassaku_b200 import _C
 
 
+def stamp_segments(lay, B: int, n_slots: int, stamp_users, stamp_items):
+    """(segments, stamps_users | None, stamps_items | None) for a batch of B samples and n_slots item slots: the row
+    segments of arena layout `lay` whose untouched rows skip the gradient traffic — only a table the batch covers
+    sparsely (otherwise the plain streaming pass is at least as fast and no marking launch is spent)."""
+    su = stamp_users if 4 * B <= lay.n_users else None
+    si = stamp_items if n_slots <= lay.n_items else None
+    segs = []
+    if su is not None:
+        segs.append((lay.off_U, lay.n_users, lay.ld, su))
+    if si is not None:
+        segs.append((lay.off_V, lay.n_items, lay.ld, si))
+    return tuple(segs), su, si
+
+
 class DenseAdam(torch.optim.Optimizer):
     """`decoupled=True` -> torch.optim.AdamW(lr, weight_decay); False -> torch.optim.Adam(lr, weight_decay) (L2).
     Defaults as torch: betas (0.9, 0.999), eps 1e-8, AdamW weight_decay default is whatever the caller passes
@@ -58,17 +72,10 @@ class DenseAdam(torch.optim.Optimizer):
         if self.mode == 'lazy':
             _C.mark_touched(u_idxs, i_idxs, lay.n_users, lay.n_items, self.touched_users, self.touched_items)
             return
-        B, n_slots = int(u_idxs.numel()), int(i_idxs.numel())
-        su = self.stamp_users if 4 * B <= lay.n_users else None
-        si = self.stamp_items if n_slots <= lay.n_items else None
-        segs = []
-        if su is not None:
-            segs.append((lay.off_U, lay.n_users, lay.ld, su))
-        if si is not None:
-            segs.append((lay.off_V, lay.n_items, lay.ld, si))
+        segs, su, si = stamp_segments(lay, int(u_idxs.numel()), int(i_idxs.numel()), self.stamp_users, self.stamp_items)
         if segs:
             _C.mark_batch(u_idxs, i_idxs, lay.n_users, lay.n_items, su, si, step=self.t + 1)
-        self._segments = tuple(segs)
+        self._segments = segs
 
     def _step_lazy(self, grp):
         lay, arena = self.model.layout, self.model.arena

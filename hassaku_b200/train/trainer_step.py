@@ -6,23 +6,17 @@ from hassaku_b200.train.optim import DenseAdam
 from hassaku_b200.train.rec_losses import RecommenderSystemLoss
 
 
-class FusedMFTrainStep:
-    """One training step of SGDMatrixFactorization: trainer.py:133-148 as hsk_mf_train_fused + hsk_adamw_dense."""
+class HostBatchStager:
+    """Host batches (the reference loaders) to the device: 3 rotating device staging slots filled on a copy stream, so
+    the H2D of batch s+1 overlaps the kernels of batch s.  `stage` returns (slot, u, i); record slot['free'] on the
+    compute stream after the batch's last kernel."""
 
-    def __init__(self, model, rec_loss: RecommenderSystemLoss, optimizer: DenseAdam):
-        if rec_loss.loss_kind not in _C.LOSS_KINDS:
-            raise ValueError(f'Loss {rec_loss.name} has no fused kernel')
-        self.model, self.rec_loss, self.optimizer = model, rec_loss, optimizer
-        self.kind = _C.LOSS_KINDS[rec_loss.loss_kind]
-        self.shift = float(rec_loss.neg_shift())
-        self.device = model.arena.device
-        self.loss_accum = torch.zeros(1, dtype=torch.float64, device=self.device)
-        # host batches (the reference loaders): 3 rotating device staging slots filled on a copy stream, so the H2D
-        # of batch s+1 overlaps the kernels of batch s
+    def __init__(self, device):
+        self.device = device
         self._copy_stream = None
         self._slots, self._k = [], 0
 
-    def _stage(self, u_host: torch.Tensor, i_host: torch.Tensor):
+    def stage(self, u_host: torch.Tensor, i_host: torch.Tensor):
         if self._copy_stream is None:
             self._copy_stream = torch.cuda.Stream(device=self.device)
         B, N1 = i_host.shape
@@ -42,6 +36,26 @@ class FusedMFTrainStep:
         torch.cuda.current_stream().wait_event(sl['ready'])
         return sl, sl['u'][:B], sl['i'][:B]
 
+    def device_batch(self, u_idxs: torch.Tensor, i_idxs: torch.Tensor):
+        """(slot or None, u, i): device batches pass through as int64, host batches are staged."""
+        if u_idxs.is_cuda and i_idxs.is_cuda:
+            return None, u_idxs.to(self.device, torch.int64).contiguous(), i_idxs.to(self.device, torch.int64).contiguous()
+        return self.stage(u_idxs, i_idxs)
+
+
+class FusedMFTrainStep:
+    """One training step of SGDMatrixFactorization: trainer.py:133-148 as hsk_mf_train_fused + hsk_adamw_dense."""
+
+    def __init__(self, model, rec_loss: RecommenderSystemLoss, optimizer: DenseAdam):
+        if rec_loss.loss_kind not in _C.LOSS_KINDS:
+            raise ValueError(f'Loss {rec_loss.name} has no fused kernel')
+        self.model, self.rec_loss, self.optimizer = model, rec_loss, optimizer
+        self.kind = _C.LOSS_KINDS[rec_loss.loss_kind]
+        self.shift = float(rec_loss.neg_shift())
+        self.device = model.arena.device
+        self.loss_accum = torch.zeros(1, dtype=torch.float64, device=self.device)
+        self._stager = HostBatchStager(self.device)
+
     def __call__(self, u_idxs: torch.Tensor, i_idxs: torch.Tensor, loss_out: torch.Tensor = None):
         """Enqueue one step.  `loss_out` (fp64 [1], device) receives this batch's mean loss added to it; by default
         the epoch accumulator is used."""
@@ -49,13 +63,8 @@ class FusedMFTrainStep:
             self._step(u_idxs, i_idxs, loss_out)
 
     def _step(self, u_idxs, i_idxs, loss_out):
-        slot = None
-        if u_idxs.is_cuda and i_idxs.is_cuda:
-            u = u_idxs.to(self.device, torch.int64).contiguous()
-            i = i_idxs.to(self.device, torch.int64).contiguous()
-        else:
-            slot, u, i = self._stage(u_idxs, i_idxs)
-        loss = self.loss_accum if loss_out is None else loss_out
+        slot, u, i = self._stager.device_batch(u_idxs, i_idxs)
+        loss =self.loss_accum if loss_out is None else loss_out
         if determinism.enabled():
             scratch = determinism.scratch(self, _C.det_scratch_bytes(i.shape[0], i.shape[1], self.model.layout.ld),
                                           self.device)

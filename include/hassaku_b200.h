@@ -396,6 +396,37 @@ HSK_API int hsk_adamw_consts(double lr, double beta1, double beta2, double eps, 
 HSK_API int hsk_adamw_dense_graph(float* p, float* m, float* v, float* g, int64_t n, const float* consts_dev,
                                   int decoupled_decay, int adam_l2, int zero_grad, hsk_stream_t stream);
 
+/* ==== trial pack: M models of one shape (a hyperparameter sweep) trained by one launch per kernel ====================
+ * The M parameter arenas are the rows of one [M, trial_stride] fp32 allocation (m, v and the gradient arena likewise):
+ * trial j's tables are trial 0's tables + j * trial_stride elements.  trial_stride % 4 == 0, so with trial 0's tables
+ * 16-byte aligned every trial's are.  `active` (device int32 [n_active]) lists the trials a launch works on; one grid
+ * dimension walks it, so an inactive trial costs no CTA and none of its memory is read or written.  An entry outside
+ * [0, n_trials) sets HSK_STATUS_BAD_INDEX in `status` and that entry's work is skipped.  n_active <= 65535.
+ *   hsk_mf_train_fused_pack  hsk_mf_train_fused for every active trial on ONE shared batch u_idx / i_idx: t / g = trial
+ *       0's parameter / gradient tables, loss_accum [n_trials] fp64 (trial j adds its batch-mean loss to loss_accum[j]).
+ *       Kernel and item-slot split follow HSK_TRAIN_AUTO's rules applied to n_active * B samples, with the
+ *       register-gather kernel wherever AUTO would take the bulk-copy ring.  Scores / dscores are not written.
+ *   hsk_adamw_pack  hsk_adamw_dense (arith 0, gradient zeroed) for every active trial, in one streaming pass:
+ *       consts_dev [n_trials, 8] fp32 = each trial's hsk_adamw_consts for this step (16-byte aligned).  adam_l2 = 0:
+ *       AdamW; 1: Adam(L2).  A trial whose wd entry is 0 gets no weight-decay term, as torch does for wd == 0 (torch tests
+ *       the double: the two agree unless 0 < |wd| < 2^-150).  n_segments > 0 is the row-stamped form of
+ *       hsk_adamw_dense_rows: `segments` are offsets inside ONE trial's row (0 <= offset, end <= trial_stride), the stamp
+ *       arrays are shared by every trial (every trial saw the same batch) and `step` (>= 1) selects the stamp; outside
+ *       the segments the row takes the dense path in the same launch.  Bitwise identical to hsk_adamw_dense /
+ *       hsk_adamw_dense_rows with arith 0 per trial.
+ *   hsk_adamw_consts_table  host: out [n_steps, n_trials, 8] = hsk_adamw_consts(lr[j], ..., weight_decay[j], first_step +
+ *       s) for every step s and trial j (one table per epoch: no per-step host work or copy). */
+HSK_API int hsk_mf_train_fused_pack(const hsk_mf_tables* t, const hsk_mf_tables* g, int64_t trial_stride, int n_trials,
+                                    const int32_t* active, int n_active, const int64_t* u_idx, const int64_t* i_idx, int B,
+                                    int N1, int loss_kind, float neg_shift, double* loss_accum /* [n_trials] */,
+                                    int32_t* status, hsk_stream_t stream);
+HSK_API int hsk_adamw_pack(float* p, float* m, float* v, float* g, int64_t trial_stride, int n_trials, const int32_t* active,
+                           int n_active, const float* consts_dev, const hsk_row_segment* segments /* host, nullable */,
+                           int n_segments /* <= 4 */, int64_t step, int adam_l2, int32_t* status, hsk_stream_t stream);
+HSK_API int hsk_adamw_consts_table(const double* lr /* host [n_trials] */, const double* weight_decay /* host [n_trials] */,
+                                   int n_trials, double beta1, double beta2, double eps, int64_t first_step, int n_steps,
+                                   float* out /* host [n_steps, n_trials, 8] */);
+
 /* ==== deterministic mode (hsk_det.cu): bitwise-reproducible training / evaluation reductions ========================
  * What the Python layer runs under torch.use_deterministic_algorithms(True).  The batch is grouped by row (stable radix
  * sort of the item ids of the B * N1 slots and of the user ids of the B samples) and every touched row is produced by ONE
