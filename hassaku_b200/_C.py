@@ -93,7 +93,7 @@ def _declare(lib):
         'hsk_adamw_dense_rows': (i32, [vp, vp, vp, vp, i64, C.POINTER(RowSegment), i32, f64, f64, f64, f64, f64, i64, vp, vp, i32, i32, vp]),
         'hsk_rescore_topk': (i32, [T, vp, i32, i64, i64, vp, vp, i32, i32, vp, vp, vp, vp]),
         'hsk_rescore_scores': (i32, [T, vp, i32, i64, i64, vp, i32, vp, vp, vp]),
-        'hsk_topk_combine': (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp]),
+        'hsk_topk_combine': (i32, [vp, vp, vp, i32, i32, i32, i32, vp, vp, vp]),
         'hsk_shard_block_rows': (i64, [i32, i32]),
         'hsk_route_scratch_bytes': (i64, [i64, i32]),
         'hsk_route_items': (i32, [vp, i64, i64, i32, i32, i32, vp, vp, vp, vp, i64, vp, vp]),
@@ -711,16 +711,21 @@ def rescore_scores(tables: MfTables, u_rows, cand_ids, out_scores, id_offset: in
                                         out_scores.data_ptr(), _ptr(status), st), 'hsk_rescore_scores')
 
 
-def topk_combine(scores, ids, k: int, out_scores, out_ids):
-    """scores [G, rows, n_cand] (finite where shard g owns the item), ids [rows, n_cand] -> the k best per row."""
+def topk_combine(scores, ids, k: int, out_scores, out_ids, cand_scores=None):
+    """scores [G, rows, n_cand] (finite where shard g owns the item), ids [rows, n_cand] -> the k best per row;
+    cand_scores [rows, n_cand] (the merged low-precision scores): -inf marks an excluded item, which stays -inf."""
     _req(scores, torch.float32, 'scores'); _req(ids, torch.int32, 'ids')
     _req(out_scores, torch.float32, 'out_scores'); _req(out_ids, torch.int32, 'out_ids')
     G, rows, n_cand = scores.shape
     if tuple(ids.shape) != (rows, n_cand) or tuple(out_scores.shape) != (rows, k) or tuple(out_ids.shape) != (rows, k):
         raise HskError('topk_combine: ids must be [rows, n_cand], outputs [rows, k]')
-    with _on_device_of(scores, ids, out_scores, out_ids) as st:
-        _check(lib().hsk_topk_combine(scores.data_ptr(), ids.data_ptr(), G, rows, n_cand, k, out_scores.data_ptr(),
-                                      out_ids.data_ptr(), st), 'hsk_topk_combine')
+    if cand_scores is not None:
+        _req(cand_scores, torch.float32, 'cand_scores')
+        if cand_scores.shape != ids.shape:
+            raise HskError('topk_combine: cand_scores must have the shape of ids')
+    with _on_device_of(scores, ids, cand_scores, out_scores, out_ids) as st:
+        _check(lib().hsk_topk_combine(scores.data_ptr(), ids.data_ptr(), _ptr(cand_scores), G, rows, n_cand, k,
+                                      out_scores.data_ptr(), out_ids.data_ptr(), st), 'hsk_topk_combine')
 
 
 def topk_merge(scores, ids, out_scores, out_ids):

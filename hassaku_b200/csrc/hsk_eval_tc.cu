@@ -257,8 +257,16 @@ eval_topk_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                         s_tau[rr] = ntau; s_taukey[rr] = ntaukey;
                     }
                     if (last) {
+                        int n_final = total;
+                        if (total < a.k) {   // this split's items [t_begin, t_end) x TC_BN, local row n = global id id_offset + n * id_stride
+                            const int64_t n_lo = (int64_t)t_begin * TC_BN, n_hi = min((int64_t)t_end * TC_BN, a.n_local) - 1;
+                            n_final = tc_fill_excluded<2>(lp, total, a.k, lane, a.excl_indices, s_exlo[rr], s_exhi[rr],
+                                                          (uint32_t)(a.id_offset + n_lo * a.id_stride),
+                                                          (uint32_t)(a.id_offset + n_hi * a.id_stride),
+                                                          [&](uint32_t id) { return ((int64_t)id - a.id_offset) % a.id_stride == 0; });
+                        }
                         uint64_t keys[kKeysPerLane];
-                        tc_final_sort<2>(lp, total, a.k, lane, keys);
+                        tc_final_sort<2>(lp, n_final, a.k, lane, keys);
                         if (a.n_splits == 1) {
                             const int64_t orow = (int64_t)(m0 + rr) * a.k;
                             const float base = s_base[rr];

@@ -292,8 +292,44 @@ static __device__ __noinline__ int tc_cut_row(uint64_t* lp, const int* c, int k,
     return total;
 }
 
-// Final, exact: `total` <= 192 survivors dealt round-robin over the NR regions (as tc_cut_row leaves them) are sorted with
-// the 256-key network and the best k written to lp[0..k) / returned in key[] (element e = r * 32 + lane).
+// The -inf tail of a row with fewer than k admissible items (total < k survivors after the last cut): the reference ranks
+// the user's excluded items after every admissible one, at score -inf, lowest id first.  The scan never appends them, so
+// the warp walks the exclusion row [lo, hi) upwards from the first id >= id_lo and appends, after the survivors in the
+// round-robin layout, the first k ids that this launch covers (`covered(id)`; the walk stops past id_hi), keyed
+// make_key(-inf, id).  k of them rather than k - total keeps the result exact when admissible items score -inf too.
+// Returns the new list length (<= total + k < 256 for the final sort).
+template <int NR, class Covered>
+static __device__ __forceinline__ int tc_fill_excluded(uint64_t* lp, int total, int k, int lane, const int32_t* __restrict__ excl,
+                                                       int64_t lo, int64_t hi, uint32_t id_lo, uint32_t id_hi, Covered covered) {
+    constexpr int RC = TC_CAP / NR;
+    {   // lower bound of id_lo in the sorted row
+        int64_t a = lo, b = hi;
+        while (a < b) {
+            const int64_t mid = (a + b) >> 1;
+            if ((uint32_t)__ldg(excl + mid) < id_lo) a = mid + 1; else b = mid;
+        }
+        lo = a;
+    }
+    int added = 0;
+    for (int64_t base = lo; base < hi && added < k; base += 32) {
+        const int64_t p = base + lane;
+        const uint32_t id = p < hi ? (uint32_t)__ldg(excl + p) : 0xFFFFFFFFu;
+        const bool take = p < hi && id <= id_hi && covered(id);
+        const unsigned m = __ballot_sync(kFull, take);
+        const int pos = added + __popc(m & ((1u << lane) - 1));
+        if (take && pos < k) {
+            const int e = total + pos;
+            lp[(e % NR) * RC + e / NR] = make_key(-INFINITY, id);
+        }
+        added += __popc(m);
+        if (__any_sync(kFull, id > id_hi)) break;
+    }
+    __syncwarp();
+    return total + min(added, k);
+}
+
+// Final, exact: `total` <= 255 keys dealt round-robin over the NR regions (as tc_cut_row and tc_fill_excluded leave them)
+// are sorted with the 256-key network and the best k written to lp[0..k) / returned in key[] (element e = r * 32 + lane).
 template <int NR>
 static __device__ __noinline__ void tc_final_sort(uint64_t* lp, int total, int k, int lane, uint64_t (&key)[kKeysPerLane]) {
     constexpr int RC = TC_CAP / NR;

@@ -398,8 +398,28 @@ eval_topk_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                         s_tau[rr] = ntau; s_taukey[rr] = ntaukey;
                     }
                     if (last) {
+                        int n_final = total;
+                        if (total < a.k) {
+                            // this split's tiles [t_begin, t_end): id = id_offset + (q + n_shards * n) * id_stride for row n of
+                            // shard q, in global tile shard_tile_end[q - 1] + n / T2_BN
+                            const bool one = a.n_shards == 1;
+                            const int64_t n_hi = one ? min((int64_t)t_end * T2_BN, a.shard_rows[0]) - 1 : 0;
+                            n_final = tc_fill_excluded<NCG>(lp, total, a.k, lane, a.excl_indices, s_exlo[rr], s_exhi[rr],
+                                                            (uint32_t)(a.id_offset + (one ? (int64_t)t_begin * T2_BN * a.id_stride : 0)),
+                                                            one ? (uint32_t)(a.id_offset + n_hi * a.id_stride) : 0xFFFFFFFFu,
+                                                            [&](uint32_t id) {
+                                const int64_t rel = (int64_t)id - a.id_offset;
+                                if (rel < 0 || rel % a.id_stride != 0) return false;
+                                const int64_t j = rel / a.id_stride;
+                                const int qq = (int)(j % a.n_shards);
+                                const int64_t n = j / a.n_shards;
+                                if (n >= a.shard_rows[qq]) return false;
+                                const int64_t gt = (qq ? a.shard_tile_end[qq - 1] : 0) + n / T2_BN;
+                                return gt >= t_begin && gt < t_end;
+                            });
+                        }
                         uint64_t keys[kKeysPerLane];
-                        tc_final_sort<NCG>(lp, total, a.k, lane, keys);
+                        tc_final_sort<NCG>(lp, n_final, a.k, lane, keys);
                         if (a.n_splits == 1) {
                             const int64_t orow = (int64_t)(m0 + rr) * a.k;
                             const float base = s_base[rr];

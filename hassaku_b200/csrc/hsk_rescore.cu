@@ -222,9 +222,11 @@ extern "C" int hsk_rescore_scores(const hsk_mf_tables* t, const int64_t* u_rows,
 
 // ---- item-sharded evaluation, last step: the owner of a user row holds the merged candidate ids [rows, n_cand] and, from
 // every shard, the positional fp32 scores [G, rows, n_cand] (finite only where that shard owns the item): the score of a
-// candidate is the maximum over the shards; the k best by (score desc, id asc) are the row's result.
+// candidate is the maximum over the shards; the k best by (score desc, id asc) are the row's result.  A candidate whose
+// merged low-precision score (cand_scores, nullable) is -inf is an excluded item of the row's -inf tail: it stays -inf.
 namespace hsk {
-__global__ void __launch_bounds__(256) topk_combine_kernel(const float* __restrict__ scores, const int32_t* __restrict__ ids, int G,
+__global__ void __launch_bounds__(256) topk_combine_kernel(const float* __restrict__ scores, const int32_t* __restrict__ ids,
+                                                           const float* __restrict__ cand_scores, int G,
                                                            int rows, int n_cand, int k, float* __restrict__ out_s,
                                                            int32_t* __restrict__ out_i) {
     const int lane = threadIdx.x & 31;
@@ -239,7 +241,8 @@ __global__ void __launch_bounds__(256) topk_combine_kernel(const float* __restri
             const int32_t id = ids[(int64_t)row * n_cand + c];
             if (id >= 0) {
                 float sc = -INFINITY;
-                for (int q = 0; q < G; ++q) sc = fmaxf(sc, scores[((int64_t)q * rows + row) * n_cand + c]);
+                if (!cand_scores || cand_scores[(int64_t)row * n_cand + c] != -INFINITY)
+                    for (int q = 0; q < G; ++q) sc = fmaxf(sc, scores[((int64_t)q * rows + row) * n_cand + c]);
                 key[r] = make_key(sc, (uint32_t)id);
             }
         }
@@ -256,11 +259,11 @@ __global__ void __launch_bounds__(256) topk_combine_kernel(const float* __restri
 }
 }  // namespace hsk
 
-extern "C" int hsk_topk_combine(const float* scores, const int32_t* ids, int G, int rows, int n_cand, int k, float* out_scores,
-                                int32_t* out_ids, hsk_stream_t stream) {
+extern "C" int hsk_topk_combine(const float* scores, const int32_t* ids, const float* cand_scores, int G, int rows, int n_cand,
+                                int k, float* out_scores, int32_t* out_ids, hsk_stream_t stream) {
     HSK_REQUIRE(scores && ids && out_scores && out_ids, "hsk_topk_combine: null pointer");
     HSK_REQUIRE(G >= 1 && rows >= 0 && n_cand >= 1 && n_cand <= kRescoreMax && k >= 1 && k <= n_cand, "hsk_topk_combine: bad sizes");
     if (rows == 0) return HSK_OK;
-    topk_combine_kernel<<<(rows + 7) / 8, 256, 0, as_stream(stream)>>>(scores, ids, G, rows, n_cand, k, out_scores, out_ids);
+    topk_combine_kernel<<<(rows + 7) / 8, 256, 0, as_stream(stream)>>>(scores, ids, cand_scores, G, rows, n_cand, k, out_scores, out_ids);
     return check_launch("hsk_topk_combine");
 }

@@ -16,8 +16,10 @@ constexpr int kCap = 256;          // candidate-list capacity per row
 constexpr int kKeysPerLane = 8;    // kCap / 32
 constexpr int kMaxK = 128;         // largest supported k (K_VALUES max is 100, eval/eval.py:20)
 
+// -0 is mapped to +0 first: the two compare equal, so they are one score and tie by item id
 __device__ __forceinline__ uint32_t orderable(float f) {
     uint32_t u = __float_as_uint(f);
+    u = (u == 0x80000000u) ? 0u : u;
     return u ^ ((u >> 31) ? 0xFFFFFFFFu : 0x80000000u);
 }
 __device__ __forceinline__ float from_orderable(uint32_t o) {

@@ -704,7 +704,7 @@ class ShardedMF:
                     t = _C.make_tables(b['all_rows'][:, :lay.d], Vw, ub, Ib, Gb, lay.d)
                     _C.rescore_scores(t, u_rows, b['all_mci'], b['sc'], id_offset=r, id_stride=G, status=self.status)
                     self._a2a(b['recv_sc'], b['sc'].view(G, bs, kc))
-                    _C.topk_combine(b['recv_sc'], b['mci'], k, b['ms'], b['mi'])
+                    _C.topk_combine(b['recv_sc'], b['mci'], k, b['ms'], b['mi'], cand_scores=b['mcs'])
                 else:
                     self._a2a(b['recv_s'], b['top_s'].view(G, bs, k))
                     self._a2a(b['recv_i'], b['top_i'].view(G, bs, k))

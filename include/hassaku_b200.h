@@ -298,7 +298,9 @@ HSK_API int hsk_eval_topk(const hsk_mf_tables* t, const int64_t* u_idx, const in
  * row-major, bf16 (HSK_PREC_BF16) or tf32-rounded fp32 (HSK_PREC_TF32), zero padded to kpad = hsk_eval_tc_kpad(d, prec)
  * — build them with hsk_pack_rows (row_idx = u_idx gathers the batch; row_idx = NULL packs a whole table).
  * Biases stay fp32 and are added in the epilogue (Ub is the user-bias TABLE, indexed by u_idx).  Everything else as
- * hsk_eval_topk.  Supports kpad * element size <= 1024 bytes (d <= 512 bf16, d <= 256 tf32). */
+ * hsk_eval_topk, including the tail: a user with fewer than k admissible items gets them first, then the ids of the
+ * user's exclusion row at score -inf, lowest id first, then id -1 / score -inf once both run out.
+ * Supports kpad * element size <= 1024 bytes (d <= 512 bf16, d <= 256 tf32). */
 HSK_API int hsk_eval_tc_kpad(int d, int precision);
 HSK_API int hsk_pack_rows(const float* src, int ld, int d, const int64_t* row_idx /* nullable */, int64_t n_out, int64_t n_src,
                           void* dst, int kpad, int precision, int32_t* status, hsk_stream_t stream);
@@ -338,12 +340,14 @@ HSK_API int hsk_rescore_topk(const hsk_mf_tables* t, const int64_t* u_rows, int 
  *   hsk_rescore_scores  positional: out_scores[r, c] = the fp32 score of cand_ids[r, c] if this shard owns it
  *                       ((id - id_offset) % id_stride == 0), else -inf (ids of other shards are expected here);
  *   hsk_topk_combine    on the row's owner: scores [G, rows, n_cand] from all shards + the merged ids [rows, n_cand] ->
- *                       candidate score = max over shards, then the k best ordered like hsk_eval_topk. */
+ *                       candidate score = max over shards, then the k best ordered like hsk_eval_topk.  cand_scores
+ *                       (nullable, [rows, n_cand]: the merged low-precision scores): -inf marks an excluded item of
+ *                       the tail, which stays -inf as in hsk_rescore_topk. */
 HSK_API int hsk_rescore_scores(const hsk_mf_tables* t, const int64_t* u_rows, int Be, int64_t id_offset, int64_t id_stride,
                                const int32_t* cand_ids, int n_cand, float* out_scores /* [Be, n_cand] */, int32_t* status,
                                hsk_stream_t stream);
-HSK_API int hsk_topk_combine(const float* scores, const int32_t* ids, int G, int rows, int n_cand, int k, float* out_scores,
-                             int32_t* out_ids, hsk_stream_t stream);
+HSK_API int hsk_topk_combine(const float* scores, const int32_t* ids, const float* cand_scores /* nullable */, int G, int rows,
+                             int n_cand, int k, float* out_scores, int32_t* out_ids, hsk_stream_t stream);
 
 /* ---- merge of G per-shard top-k lists (item-sharded evaluation: all-gather, then this) --------------------------
  * scores/ids: [G, rows, k] (id < 0 = empty slot) -> out [rows, k], same ordering rule as hsk_eval_topk. */

@@ -70,7 +70,7 @@ def main():
         timed('a2a scores', lambda: coll(dist.all_to_all_single, rsc, sc.view(G, bs, kc)))
         if G == 1:
             rsc.copy_(sc.view(G, bs, kc))
-        timed('topk_combine', lambda: _C.topk_combine(rsc, mci, k, ms, mi))
+        timed('topk_combine', lambda: _C.topk_combine(rsc, mci, k, ms, mi, cand_scores=mcs))
     torch.cuda.synchronize()
     if rank == 0:
         tot = 0.0
