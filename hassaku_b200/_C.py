@@ -128,6 +128,11 @@ def _declare(lib):
         'hsk_mf_train_fused_pack': (i32, [T, T, i64, i32, vp, i32, vp, vp, i32, i32, i32, f32, vp, vp, vp]),
         'hsk_adamw_pack': (i32, [vp, vp, vp, vp, i64, i32, vp, i32, vp, C.POINTER(RowSegment), i32, i64, i32, vp, vp]),
         'hsk_adamw_consts_table': (i32, [vp, vp, i32, f64, f64, f64, i64, i32, vp]),
+        'hsk_eval_topk_pack_scratch_bytes': (i64, [i32, i64, i32, i32]),
+        'hsk_eval_topk_pack': (i32, [T, i64, i32, vp, i32, vp, i32, vp, vp, i32, vp, vp, vp, i64, vp, vp]),
+        'hsk_rank_metrics_pack': (i32, [vp, i32, i32, C.POINTER(C.c_int), i32, vp, vp, vp, vp, i32, vp, i32, vp, i32, vp, vp, vp,
+                                        vp, vp]),
+        'hsk_rank_metrics_sums_det_pack': (i32, [vp, i32, i32, i32, vp, vp, i32, i32, vp, i32, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -847,3 +852,73 @@ def rank_metrics_sums_det(per_user, u_idx, sums, user_group=None, n_groups=0):
     with _on_device_of(per_user, u_idx, sums, user_group) as st:
         _check(lib().hsk_rank_metrics_sums_det(per_user.data_ptr(), Be, n_ks, u_idx.data_ptr(), _ptr(user_group), n_groups,
                                                sums.data_ptr(), st), 'hsk_rank_metrics_sums_det')
+
+
+# ---- packed validation: every active trial of a pack on one shared user batch ----
+def eval_topk_pack_scratch_bytes(Be: int, n_items: int, k: int, n_active: int) -> int:
+    return int(lib().hsk_eval_topk_pack_scratch_bytes(Be, n_items, k, n_active))
+
+
+def eval_topk_pack(tables: MfTables, trial_stride: int, n_trials: int, active, u_idx, k: int, top_scores, top_ids, scratch,
+                   excl_indptr=None, excl_indices=None, status=None):
+    """hsk_eval_topk_pack: tables = trial 0's, trial j's at + j * trial_stride elements; top_scores / top_ids
+    [n_active, Be, k]."""
+    _req(u_idx, torch.int64, 'u_idx'); _req(active, torch.int32, 'active')
+    _req(top_scores, torch.float32, 'top_scores'); _req(top_ids, torch.int32, 'top_ids')
+    if excl_indptr is not None:
+        _req(excl_indptr, torch.int64, 'excl_indptr'); _req(excl_indices, torch.int32, 'excl_indices')
+    n_active, Be = active.numel(), u_idx.numel()
+    for name, t in (('top_scores', top_scores), ('top_ids', top_ids)):
+        if t.numel() != n_active * Be * k:
+            raise HskError(f'{name} must be [n_active, Be, k] = [{n_active}, {Be}, {k}]')
+    with _on_device_of(u_idx, active, top_scores, top_ids, scratch, excl_indptr, excl_indices, status) as st:
+        _check(lib().hsk_eval_topk_pack(C.byref(tables), trial_stride, n_trials, active.data_ptr(), n_active, u_idx.data_ptr(), Be,
+                                        _ptr(excl_indptr), _ptr(excl_indices), k, top_scores.data_ptr(), top_ids.data_ptr(),
+                                        scratch.data_ptr(), _scratch_bytes(scratch), _ptr(status), st), 'hsk_eval_topk_pack')
+
+
+def rank_metrics_pack(top_ids, ks, u_idx, lab_indptr, lab_indices, discount, active, sums, counts, user_group=None,
+                      n_groups=0, per_user=None, status=None):
+    """hsk_rank_metrics_pack: top_ids [n_active, Be, k_max]; sums fp64 [n_trials, 1 + n_groups, n_ks, 3], counts int64
+    [n_trials, 1 + n_groups]; per_user (optional) [n_active, Be, n_ks, 3]."""
+    _req(top_ids, torch.int32, 'top_ids'); _req(u_idx, torch.int64, 'u_idx'); _req(active, torch.int32, 'active')
+    _req(lab_indptr, torch.int64, 'lab_indptr'); _req(lab_indices, torch.int32, 'lab_indices')
+    _req(discount, torch.float32, 'discount'); _req(sums, torch.float64, 'sums'); _req(counts, torch.int64, 'counts')
+    if user_group is not None:
+        _req(user_group, torch.int32, 'user_group')
+    if per_user is not None:
+        _req(per_user, torch.float32, 'per_user')
+    n_active, Be, k_max = top_ids.shape
+    if n_active != active.numel():
+        raise HskError(f'top_ids holds {n_active} trials, active lists {active.numel()}')
+    n_trials = sums.shape[0]
+    if sums.shape != (n_trials, 1 + n_groups, len(ks), 3) or counts.shape != (n_trials, 1 + n_groups):
+        raise HskError(f'sums / counts must be [n_trials, 1 + n_groups, n_ks, 3] / [n_trials, 1 + n_groups] with n_groups = '
+                       f'{n_groups}, n_ks = {len(ks)}')
+    if per_user is not None and per_user.shape != (n_active, Be, len(ks), 3):
+        raise HskError(f'per_user must be [n_active, Be, n_ks, 3] = [{n_active}, {Be}, {len(ks)}, 3]')
+    with _on_device_of(top_ids, u_idx, active, lab_indptr, lab_indices, discount, sums, counts, user_group, per_user,
+                       status) as st:
+        _check(lib().hsk_rank_metrics_pack(top_ids.data_ptr(), Be, k_max, _ks_array(ks), len(ks), u_idx.data_ptr(),
+                                           lab_indptr.data_ptr(), lab_indices.data_ptr(), _ptr(user_group), n_groups,
+                                           discount.data_ptr(), n_trials, active.data_ptr(), n_active, _ptr(per_user),
+                                           sums.data_ptr(), counts.data_ptr(), _ptr(status), st), 'hsk_rank_metrics_pack')
+
+
+def rank_metrics_sums_det_pack(per_user, u_idx, batch: int, active, sums, user_group=None, n_groups=0, status=None):
+    """hsk_rank_metrics_sums_det_pack: sums [n_trials, 1 + n_groups, n_ks, 3] += per trial, batch by batch in order, the
+    fixed-order sums of per_user [n_active, Be, n_ks, 3]."""
+    _req(per_user, torch.float32, 'per_user'); _req(u_idx, torch.int64, 'u_idx'); _req(active, torch.int32, 'active')
+    _req(sums, torch.float64, 'sums')
+    if user_group is not None:
+        _req(user_group, torch.int32, 'user_group')
+    n_active, Be, n_ks, _ = per_user.shape
+    if n_active != active.numel():
+        raise HskError(f'per_user holds {n_active} trials, active lists {active.numel()}')
+    n_trials = sums.shape[0]
+    if sums.shape != (n_trials, 1 + n_groups, n_ks, 3):
+        raise HskError(f'sums must be [n_trials, 1 + n_groups, n_ks, 3] with n_groups = {n_groups}, n_ks = {n_ks}')
+    with _on_device_of(per_user, u_idx, active, sums, user_group, status) as st:
+        _check(lib().hsk_rank_metrics_sums_det_pack(per_user.data_ptr(), Be, batch, n_ks, u_idx.data_ptr(), _ptr(user_group),
+                                                    n_groups, n_trials, active.data_ptr(), n_active, sums.data_ptr(),
+                                                    _ptr(status), st), 'hsk_rank_metrics_sums_det_pack')

@@ -9,6 +9,7 @@
 //                              per-sample fp64 loss), then the scatter above and a fixed-order loss sum
 //   hsk_rec_loss_det           hsk_rec_loss with the per-row losses summed in a fixed order
 //   hsk_rank_metrics_sums_det  fixed-order sum of per-user metric rows into the per-group sums
+//   hsk_rank_metrics_sums_det_pack  the same for every active trial of a trial pack, batch by batch
 //
 // ORDER CONTRACT (restated by oracle/det_oracle.py, which reproduces every gradient bit in numpy float32).
 //   Slot s = b * N1 + j.  Item side: the n = B * N1 slots are stably sorted by item id, giving positions P = 0 .. n-1
@@ -538,32 +539,29 @@ __global__ void __launch_bounds__(256) det_loss_sum_kernel(const double* __restr
 __global__ void __launch_bounds__(256) det_metric_sums_kernel(const float* __restrict__ per_user, int Be, int n_cells,
                                                               const int64_t* __restrict__ u_idx, const int32_t* __restrict__ group,
                                                               int n_groups, double* sums) {
-    constexpr int kMaxCells = 24;   // n_ks <= 8 cut-offs x 3 metrics
-    __shared__ double sm[256];
-    const int g = blockIdx.x;
-    double acc[kMaxCells];
-#pragma unroll
-    for (int c = 0; c < kMaxCells; ++c) acc[c] = 0.0;
-    for (int r = threadIdx.x; r < Be; r += 256) {
-        if (g > 0) {
-            const int gr = group[u_idx[r]];
-            if (gr != g - 1 || gr >= n_groups) continue;
-        }
-#pragma unroll
-        for (int c = 0; c < kMaxCells; ++c)
-            if (c < n_cells) acc[c] = __dadd_rn(acc[c], (double)per_user[(int64_t)r * n_cells + c]);
+#include "hsk_det_metric_sums_body.inc"
+}
+
+// trial pack (hsk_rank_metrics_sums_det_pack): gridDim.y walks the active trials; per trial the rows are cut into batches of
+// `batch` and each batch is added by the body above, in order, into the trial's sums
+__global__ void __launch_bounds__(256) det_metric_sums_pack_kernel(const float* __restrict__ per_user_all, int Be_all, int batch,
+                                                                   int n_cells, const int64_t* __restrict__ u_all,
+                                                                   const int32_t* __restrict__ group, int n_groups, int groups,
+                                                                   const int32_t* __restrict__ active, int n_trials,
+                                                                   double* sums_all, int32_t* status) {
+    const int jt = active[blockIdx.y];
+    if (jt < 0 || jt >= n_trials) {
+        if (threadIdx.x == 0 && status) atomicOr(status, HSK_STATUS_BAD_INDEX);
+        return;
     }
-#pragma unroll
-    for (int c = 0; c < kMaxCells; ++c) {
-        if (c >= n_cells) break;
-        sm[threadIdx.x] = acc[c];
-        __syncthreads();
-        for (int w = 128; w > 0; w >>= 1) {
-            if (threadIdx.x < w) sm[threadIdx.x] = __dadd_rn(sm[threadIdx.x], sm[threadIdx.x + w]);
-            __syncthreads();
+    double* sums = sums_all + (int64_t)jt * (1 + groups) * n_cells;
+    for (int b0 = 0; b0 < Be_all; b0 += batch) {
+        const float* __restrict__ per_user = per_user_all + ((int64_t)blockIdx.y * Be_all + b0) * n_cells;
+        const int Be = min(batch, Be_all - b0);
+        const int64_t* __restrict__ u_idx = u_all + b0;
+        {
+#include "hsk_det_metric_sums_body.inc"
         }
-        if (threadIdx.x == 0) sums[(int64_t)g * n_cells + c] = __dadd_rn(sums[(int64_t)g * n_cells + c], sm[0]);
-        __syncthreads();
     }
 }
 
@@ -700,4 +698,21 @@ extern "C" int hsk_rank_metrics_sums_det(const float* per_user, int Be, int n_ks
     const int G = user_group ? n_groups : 0;
     det_metric_sums_kernel<<<1 + G, 256, 0, as_stream(stream)>>>(per_user, Be, n_ks * 3, u_idx, user_group, G, sums);
     return check_launch("hsk_rank_metrics_sums_det");
+}
+
+extern "C" int hsk_rank_metrics_sums_det_pack(const float* per_user, int Be, int batch, int n_ks, const int64_t* u_idx,
+                                              const int32_t* user_group, int n_groups, int n_trials, const int32_t* active,
+                                              int n_active, double* sums, int32_t* status, hsk_stream_t stream) {
+    HSK_REQUIRE(per_user && u_idx && sums, "hsk_rank_metrics_sums_det_pack: null pointer");
+    HSK_REQUIRE(n_ks >= 1 && n_ks <= 8 && n_groups >= 0 && Be >= 0 && batch >= 1,
+                "hsk_rank_metrics_sums_det_pack: need 1 <= n_ks <= 8, batch >= 1");
+    HSK_REQUIRE(n_trials >= 1 && n_active >= 0 && n_active <= n_trials && n_active <= 65535,
+                "hsk_rank_metrics_sums_det_pack: need 0 <= n_active <= n_trials, n_trials >= 1, n_active <= 65535 (n_trials=%d n_active=%d)",
+                n_trials, n_active);
+    HSK_REQUIRE(n_active == 0 || active, "hsk_rank_metrics_sums_det_pack: active is null");
+    if (Be == 0 || n_active == 0) return HSK_OK;
+    const int G = user_group ? n_groups : 0;
+    det_metric_sums_pack_kernel<<<dim3(1 + G, n_active), 256, 0, as_stream(stream)>>>(per_user, Be, batch, n_ks * 3, u_idx, user_group,
+                                                                                    G, n_groups, active, n_trials, sums, status);
+    return check_launch("hsk_rank_metrics_sums_det_pack");
 }

@@ -7,6 +7,7 @@
 //   hsk_topk_dense    top-k of a dense logits matrix (FullEvaluator.eval_batch's dense API, eval.py:61-63)
 //   hsk_rank_metrics  precision / recall / ndcg @ ks from top-k ids + CSR labels, per-group sums on device
 //   hsk_rank_metrics_dense   same from dense y_true rows (the reference's dense API)
+//   hsk_eval_topk_pack / hsk_rank_metrics_pack   the same two for every active trial of a trial pack in one launch
 //
 // fp32-exact scoring is a classic SIMT FFMA tile kernel (64 users x 128 items per CTA, 16-wide K chunks staged by
 // cp.async double buffering, 4x8 accumulators per thread): north_star requires bit-exact top-k ids against the fp32
@@ -73,171 +74,9 @@ __device__ __noinline__ void ev_final_sort(uint64_t* list, int n, int k, int lan
 }
 
 __global__ void __launch_bounds__(kEvalThreads, 2) eval_topk_f32_kernel(EvalArgs a) {
-    __shared__ __align__(16) float As[2][TM][KP];
-    __shared__ __align__(16) float Bs[2][TN][KP];
-    __shared__ int64_t s_uoff[TM];       // element offset of the user's row in Uw, -1 = invalid row
-    __shared__ int64_t s_ex_lo[TM], s_ex_hi[TM];
-    __shared__ float s_ubias[TM];
-    __shared__ float s_tauf[TM];
-    __shared__ uint64_t s_taukey[TM];
-    __shared__ int s_cnt[TM];
-    __shared__ int s_checked[TM];   // leading entries of the row's list already tested against the exclusion row
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int tx = tid & 15, ty = tid >> 4;
-    const int m0 = blockIdx.x * TM;
-    const int split = blockIdx.y;
-    const int t_begin = split * a.tiles_per_split;
-    const int t_end = min(a.n_tiles, t_begin + a.tiles_per_split);
-
-    if (tid < TM) {
-        const int row = m0 + tid;
-        int64_t off = -1, lo = 0, hi = 0;
-        float ub = 0.f;
-        if (row < a.Be) {
-            const int64_t u = a.u_idx[row];
-            const int64_t ur = a.u_rows ? a.u_rows[row] : u;
-            if (bad_index(u, a.n_users) || bad_index(ur, a.n_urows)) {
-                if (a.status) atomicOr(a.status, HSK_STATUS_BAD_INDEX);
-            } else {
-                off = ur * a.ld;
-                if (a.excl_indptr) { lo = a.excl_indptr[u]; hi = a.excl_indptr[u + 1]; }
-                if (a.Ub) ub = a.Ub[ur];
-            }
-        }
-        s_uoff[tid] = off; s_ex_lo[tid] = lo; s_ex_hi[tid] = hi; s_ubias[tid] = ub;
-        s_tauf[tid] = -INFINITY; s_taukey[tid] = 0ull; s_cnt[tid] = 0; s_checked[tid] = 0;
-    }
-    __syncthreads();
-
-    const float gb = a.Gb ? a.Gb[0] : 0.f;
-    const int nk = (a.ld + KC - 1) / KC;
-    const int prune_at = EV_CAP - TN;  // a tile appends at most TN keys per row
-
-    for (int t = t_begin; t < t_end; ++t) {
-        const int64_t n0 = (int64_t)t * TN;
-        float acc[4][8];
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-
-        auto load_stage = [&](int stage, int kc) {
-            const int k0 = kc * KC;
-            {   // A: 64 rows x 4 float4
-                const int r = tid >> 2, q = tid & 3;
-                const int kk = k0 + q * 4;
-                const int64_t off = s_uoff[r];
-                const bool ok = off >= 0 && kk < a.ld;
-                cp_async16(&As[stage][r][q * 4], ok ? (a.Uw + off + kk) : a.Uw, ok ? 16 : 0);
-            }
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {  // B: 128 rows x 4 float4
-                const int idx = tid + kEvalThreads * h;
-                const int r = idx >> 2, q = idx & 3;
-                const int kk = k0 + q * 4;
-                const int64_t n = n0 + r;
-                const bool ok = n < a.n_local && kk < a.ld;
-                cp_async16(&Bs[stage][r][q * 4], ok ? (a.Vw + n * a.ld + kk) : a.Vw, ok ? 16 : 0);
-            }
-            cp_async_commit();
-        };
-
-        load_stage(0, 0);
-        for (int kc = 0; kc < nk; ++kc) {
-            const int st = kc & 1;
-            if (kc + 1 < nk) { load_stage(st ^ 1, kc + 1); cp_async_wait<1>(); } else { cp_async_wait<0>(); }
-            __syncthreads();
-#pragma unroll
-            for (int kk = 0; kk < KC; kk += 4) {
-                float4 av[4], bv[8];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) av[i] = *reinterpret_cast<const float4*>(&As[st][ty + 16 * i][kk]);
-#pragma unroll
-                for (int j = 0; j < 8; ++j) bv[j] = *reinterpret_cast<const float4*>(&Bs[st][tx + 16 * j][kk]);
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        acc[i][j] = fmaf(av[i].x, bv[j].x, acc[i][j]);
-                        acc[i][j] = fmaf(av[i].y, bv[j].y, acc[i][j]);
-                        acc[i][j] = fmaf(av[i].z, bv[j].z, acc[i][j]);
-                        acc[i][j] = fmaf(av[i].w, bv[j].w, acc[i][j]);
-                    }
-            }
-            __syncthreads();
-        }
-
-        // ---- epilogue: biases, threshold filter; the rare survivors get the exclusion test and are appended ----
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int r = ty + 16 * i;
-            if (s_uoff[r] < 0) continue;
-            const float tauf = s_tauf[r];
-            const float ub = s_ubias[r];
-            uint64_t* list = a.cand + ((int64_t)split * a.Be + (m0 + r)) * EV_CAP;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const int64_t n = n0 + tx + 16 * j;
-                if (n >= a.n_local) continue;
-                float s = acc[i][j];
-                if (a.Ub) s += ub;            // sgd_alg.py:173-178 order: user bias, item bias, global bias
-                if (a.Ib) s += __ldg(a.Ib + n);
-                if (a.Gb) s += gb;
-                if (s >= tauf) {  // raw candidate; the exclusion mask (eval.py:250-251) is applied when the list is pruned
-                    const int64_t gid = a.id_offset + n * a.id_stride;
-                    const uint64_t key = make_key(s, (uint32_t)gid);
-                    if (key > s_taukey[r]) {
-                        const int pos = atomicAdd(&s_cnt[r], 1);
-                        list[pos] = key;
-                    }
-                }
-            }
-        }
-        __syncthreads();
-        const bool last = (t + 1 == t_end);
-        for (int r = warp; r < TM; r += kEvalThreads / 32) {
-            if (s_uoff[r] < 0) {  // bad user index: leave an empty list for the merge
-                if (last && a.n_splits > 1 && m0 + r < a.Be) {
-                    uint64_t* list = a.cand + ((int64_t)split * a.Be + (m0 + r)) * EV_CAP;
-                    for (int e = lane; e < a.k; e += 32) list[e] = 0ull;
-                }
-                continue;
-            }
-            const int n = s_cnt[r];
-            if (n > prune_at || last) {
-                uint64_t* list = a.cand + ((int64_t)split * a.Be + (m0 + r)) * EV_CAP;
-                float ntau;
-                uint64_t ntaukey;
-                const int total = ev_cut(list, n, s_checked[r], a.k, lane, a.excl_indices, s_ex_lo[r], s_ex_hi[r], &ntau, &ntaukey);
-                __syncwarp();
-                if (lane == 0) {
-                    s_cnt[r] = total;
-                    s_checked[r] = total;
-                    s_taukey[r] = ntaukey;
-                    s_tauf[r] = ntau;
-                }
-                if (last) {   // exact order, once: the <= 256 survivors through the 256-key network
-                    ev_final_sort(list, total, a.k, lane);
-                    if (a.n_splits == 1) {
-                        __syncwarp();
-                        write_topk_row(list, a.k, a.out_scores + (int64_t)(m0 + r) * a.k, a.out_ids + (int64_t)(m0 + r) * a.k, lane);
-                    }
-                }
-            }
-        }
-        __syncthreads();
-    }
-    // rows with a bad user index: ids -1, scores -inf
-    if (a.n_splits == 1) {
-        for (int r = warp; r < TM; r += kEvalThreads / 32) {
-            if (m0 + r < a.Be && s_uoff[r] < 0)
-                for (int e = lane; e < a.k; e += 32) {
-                    a.out_scores[(int64_t)(m0 + r) * a.k + e] = -INFINITY;
-                    a.out_ids[(int64_t)(m0 + r) * a.k + e] = -1;
-                }
-        }
-    }
+#define EV_SPLIT_ROWS a.Be
+#include "hsk_eval_topk_body.inc"
+#undef EV_SPLIT_ROWS
 }
 
 // ---- merge of G sorted key lists per row (lists[g] at base + (g * rows + row) * stride) ----
@@ -349,75 +188,70 @@ struct MetricArgs {
 
 template <bool DENSE>
 __global__ void __launch_bounds__(256) rank_metrics_kernel(MetricArgs a) {
-    const int lane = threadIdx.x & 31;
-    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (row >= a.Be) return;
-    const int64_t u = a.u_idx[row];
-    float npos;
-    int64_t lo = 0, hi = 0;
-    if (DENSE) {
-        float sacc = 0.f;
-        for (int64_t c = lane; c < a.n_items; c += 32) sacc += a.y_true[(int64_t)row * a.n_items + c];
-        npos = warp_sum(sacc);
-    } else {
-        lo = a.lab_indptr[u]; hi = a.lab_indptr[u + 1];
-        npos = (float)(hi - lo);
-    }
-    // hit flags of the ranked list: rank r handled by lane r % 32
-    float h[4];  // k_max <= 128
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        const int r = q * 32 + lane;
-        float v = 0.f;
-        if (r < a.k_max) {
-            const int32_t id = a.top_ids[(int64_t)row * a.k_max + r];
-            if (id >= 0) {
-                if (DENSE) v = a.y_true[(int64_t)row * a.n_items + id];
-                else v = csr_contains(a.lab_indices, lo, hi, id) ? 1.f : 0.f;
-            }
-        }
-        h[q] = v;
-    }
-    const int grp = (a.user_group && a.n_groups > 0) ? a.user_group[u] : -1;
-    for (int t = 0; t < a.n_ks; ++t) {
-        const int k = a.ks[t];
-        float hits = 0.f, dcg = 0.f;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const int r = q * 32 + lane;
-            if (r < k) { hits += h[q]; dcg = fmaf(h[q], a.discount[r], dcg); }
-        }
-        hits = warp_sum(hits);
-        dcg = warp_sum(dcg);
-        if (lane == 0) {
-            // IDCG = sum of the first min(k, n+) discounts (binary relevance: y_true.topk(k).values are ones, metrics.py:94)
-            float idcg = 0.f;
-            const int kk = (int)fminf((float)k, npos);
-            for (int r = 0; r < kk; ++r) idcg += a.discount[r];
-            const float precision = hits / (float)k;
-            const float recall = npos > 0.f ? hits / npos : 0.f;           // NaN -> 0, metrics.py:28
-            const float ndcg = npos > 0.f ? fminf(dcg / idcg, 1.f) : 0.f;   // NaN -> 0, clamp, metrics.py:98-100
-            if (a.per_user) {
-                float* o = a.per_user + ((int64_t)row * a.n_ks + t) * 3;
-                o[0] = precision; o[1] = recall; o[2] = ndcg;
-            }
-            double* s0 = a.sums + (int64_t)t * 3;
-            atomicAdd(s0 + 0, (double)precision); atomicAdd(s0 + 1, (double)recall); atomicAdd(s0 + 2, (double)ndcg);
-            if (grp >= 0 && grp < a.n_groups) {
-                double* sg = a.sums + ((int64_t)(1 + grp) * a.n_ks + t) * 3;
-                atomicAdd(sg + 0, (double)precision); atomicAdd(sg + 1, (double)recall); atomicAdd(sg + 2, (double)ndcg);
-            }
-        }
-    }
-    if (lane == 0) {
-        atomicAdd(reinterpret_cast<unsigned long long*>(a.counts), 1ull);
-        if (grp >= 0 && grp < a.n_groups) atomicAdd(reinterpret_cast<unsigned long long*>(a.counts + 1 + grp), 1ull);
-    }
+#include "hsk_rank_metrics_body.inc"
 }
 
-// split plan shared by hsk_eval_topk and hsk_eval_topk_scratch_bytes
-static void eval_plan(int Be, int64_t n_local, int* n_tiles, int* tiles_per_split, int* n_splits) {
-    const int row_tiles = (Be + TM - 1) / TM;
+// ---- trial pack (hsk_eval_topk_pack, hsk_rank_metrics_pack): M models of one shape whose tables are trial 0's + j * stride
+// elements.  Kept out of EvalArgs / MetricArgs so that the single-model kernels keep their argument layout.
+struct EvalPackArgs {
+    int64_t stride;           // elements between two trials' tables
+    const int32_t* active;    // [gridDim.z] trial indices
+    int n_trials;
+    int split_rows;           // n_active * Be: rows of one split's candidate lists, laid out [split][trial][row]
+};
+
+// gridDim.z walks the active trials; x / y (row tiles, splits) as the single-model kernel over the shared user batch
+__global__ void __launch_bounds__(kEvalThreads, 2) eval_topk_f32_pack_kernel(EvalArgs a, EvalPackArgs pk) {
+    {
+        const int j = pk.active[blockIdx.z];
+        if (j < 0 || j >= pk.n_trials) {
+            if (threadIdx.x == 0 && a.status) atomicOr(a.status, HSK_STATUS_BAD_INDEX);
+            return;
+        }
+        const int64_t o = (int64_t)j * pk.stride;
+        a.Uw += o; a.Vw += o;
+        if (a.Ub) a.Ub += o;
+        if (a.Ib) a.Ib += o;
+        if (a.Gb) a.Gb += o;
+        const int64_t r0 = (int64_t)blockIdx.z * a.Be;   // this trial's first row of the [n_active * Be] outputs
+        a.cand += r0 * EV_CAP;
+        a.out_scores += r0 * a.k;
+        a.out_ids += r0 * a.k;
+    }
+#define EV_SPLIT_ROWS pk.split_rows
+#include "hsk_eval_topk_body.inc"
+#undef EV_SPLIT_ROWS
+}
+
+struct MetricPackArgs {
+    const int32_t* active;    // [gridDim.y] trial indices
+    int n_trials;
+    int groups;               // the caller's n_groups: trial j's sums / counts start at j * (1 + groups) rows
+    int32_t* status;
+};
+
+// gridDim.y walks the active trials; x as the single-model kernel over the shared user batch
+__global__ void __launch_bounds__(256) rank_metrics_pack_kernel(MetricArgs a, MetricPackArgs pk) {
+    constexpr bool DENSE = false;
+    {
+        const int j = pk.active[blockIdx.y];
+        if (j < 0 || j >= pk.n_trials) {
+            if (threadIdx.x == 0 && pk.status) atomicOr(pk.status, HSK_STATUS_BAD_INDEX);
+            return;
+        }
+        const int64_t r0 = (int64_t)blockIdx.y * a.Be;
+        a.top_ids += r0 * a.k_max;
+        if (a.per_user) a.per_user += r0 * a.n_ks * 3;
+        a.sums += (int64_t)j * (1 + pk.groups) * a.n_ks * 3;
+        a.counts += (int64_t)j * (1 + pk.groups);
+    }
+#include "hsk_rank_metrics_body.inc"
+}
+
+// split plan shared by hsk_eval_topk, hsk_eval_topk_pack and their scratch sizes: a pack multiplies the row tiles by its
+// n_active trials, so items are not split where the trials already fill the GPU
+static void eval_plan(int Be, int64_t n_local, int n_active, int* n_tiles, int* tiles_per_split, int* n_splits) {
+    const int row_tiles = (Be + TM - 1) / TM * n_active;
     const int nt = (int)((n_local + TN - 1) / TN);
     const int want = sm_count() * 2;
     int splits = 1;
@@ -445,7 +279,7 @@ using namespace hsk;
 extern "C" int64_t hsk_eval_topk_scratch_bytes(int Be, int64_t n_local_items, int k) {
     (void)k;
     int nt, tps, ns;
-    eval_plan(Be > 0 ? Be : 1, n_local_items > 0 ? n_local_items : 1, &nt, &tps, &ns);
+    eval_plan(Be > 0 ? Be : 1, n_local_items > 0 ? n_local_items : 1, 1, &nt, &tps, &ns);
     return (int64_t)ns * (Be > 0 ? Be : 1) * EV_CAP * (int64_t)sizeof(uint64_t);
 }
 
@@ -469,7 +303,7 @@ extern "C" int hsk_eval_topk(const hsk_mf_tables* t, const int64_t* u_idx, const
     a.u_idx = u_idx; a.u_rows = u_rows; a.excl_indptr = excl_indptr; a.excl_indices = excl_indices;
     a.n_users = u_rows ? n_users_global : t->n_users; a.n_urows = t->n_users; a.n_local = t->n_items; a.id_offset = id_offset; a.id_stride = id_stride;
     a.ld = t->ld; a.Be = Be; a.k = k;
-    eval_plan(Be, t->n_items, &a.n_tiles, &a.tiles_per_split, &a.n_splits);
+    eval_plan(Be, t->n_items, 1, &a.n_tiles, &a.tiles_per_split, &a.n_splits);
     const int64_t need = (int64_t)a.n_splits * Be * EV_CAP * (int64_t)sizeof(uint64_t);
     HSK_REQUIRE(scratch && scratch_bytes >= need, "hsk_eval_topk: scratch too small (%lld < %lld bytes)",
                 (long long)scratch_bytes, (long long)need);
@@ -481,6 +315,59 @@ extern "C" int hsk_eval_topk(const hsk_mf_tables* t, const int64_t* u_idx, const
     int rc = check_launch("hsk_eval_topk");
     if (rc) return rc;
     if (a.n_splits > 1) rc = launch_merge_keys(a.cand, a.n_splits, Be, EV_CAP, k, top_scores, top_ids, s, nullptr, nullptr, nullptr, 0);
+    return rc;
+}
+
+static int64_t eval_pack_scratch(int Be, int64_t n_items, int n_active, int* n_tiles, int* tps, int* n_splits) {
+    eval_plan(Be, n_items, n_active, n_tiles, tps, n_splits);
+    return (int64_t)*n_splits * n_active * Be * EV_CAP * (int64_t)sizeof(uint64_t);
+}
+
+extern "C" int64_t hsk_eval_topk_pack_scratch_bytes(int Be, int64_t n_items, int k, int n_active) {
+    (void)k;
+    int nt, tps, ns;
+    return eval_pack_scratch(Be > 0 ? Be : 1, n_items > 0 ? n_items : 1, n_active > 0 ? n_active : 1, &nt, &tps, &ns);
+}
+
+extern "C" int hsk_eval_topk_pack(const hsk_mf_tables* t, int64_t trial_stride, int n_trials, const int32_t* active, int n_active,
+                                  const int64_t* u_idx, int Be, const int64_t* excl_indptr, const int32_t* excl_indices, int k,
+                                  float* top_scores, int32_t* top_ids, void* scratch, int64_t scratch_bytes, int32_t* status,
+                                  hsk_stream_t stream) {
+    HSK_REQUIRE(t && t->Uw && t->Vw && u_idx && top_scores && top_ids, "hsk_eval_topk_pack: null pointer");
+    HSK_REQUIRE(t->d >= 1 && t->ld >= t->d && (t->ld % 4) == 0, "hsk_eval_topk_pack: need ld %% 4 == 0 (d=%d ld=%d)", t->d, t->ld);
+    HSK_REQUIRE(aligned16(t->Uw) && aligned16(t->Vw), "hsk_eval_topk_pack: tables must be 16-byte aligned");
+    HSK_REQUIRE(k >= 1 && k <= kMaxK, "hsk_eval_topk_pack: 1 <= k <= %d required (k=%d)", kMaxK, k);
+    HSK_REQUIRE(t->n_items >= 1 && Be >= 0, "hsk_eval_topk_pack: empty item table or negative batch");
+    HSK_REQUIRE(t->n_items < 0x7FFFFFFFll, "hsk_eval_topk_pack: item ids must fit int32");
+    HSK_REQUIRE((excl_indptr == nullptr) == (excl_indices == nullptr), "hsk_eval_topk_pack: exclusion CSR needs both arrays");
+    HSK_REQUIRE(n_trials >= 1 && n_active >= 0 && n_active <= n_trials && n_active <= 65535,
+                "hsk_eval_topk_pack: need 0 <= n_active <= n_trials, n_trials >= 1, n_active <= 65535 (n_trials=%d n_active=%d)",
+                n_trials, n_active);
+    HSK_REQUIRE(n_active == 0 || active, "hsk_eval_topk_pack: active is null");
+    HSK_REQUIRE(trial_stride > 0 && trial_stride % 4 == 0,
+                "hsk_eval_topk_pack: trial_stride must be a positive multiple of 4 (%lld)", (long long)trial_stride);
+    HSK_REQUIRE((int64_t)n_active * Be <= 0x7FFFFFFFll, "hsk_eval_topk_pack: n_active * Be must fit int32");
+    if (Be == 0 || n_active == 0) return HSK_OK;
+    EvalArgs a;
+    memset(&a, 0, sizeof(a));
+    a.Uw = t->Uw; a.Vw = t->Vw; a.Ub = t->Ub; a.Ib = t->Ib; a.Gb = t->Gb;
+    a.u_idx = u_idx; a.excl_indptr = excl_indptr; a.excl_indices = excl_indices;
+    a.n_users = t->n_users; a.n_urows = t->n_users; a.n_local = t->n_items; a.id_offset = 0; a.id_stride = 1;
+    a.ld = t->ld; a.Be = Be; a.k = k;
+    const int64_t need = eval_pack_scratch(Be, t->n_items, n_active, &a.n_tiles, &a.tiles_per_split, &a.n_splits);
+    HSK_REQUIRE(scratch && scratch_bytes >= need, "hsk_eval_topk_pack: scratch too small (%lld < %lld bytes)",
+                (long long)scratch_bytes, (long long)need);
+    a.cand = reinterpret_cast<uint64_t*>(scratch);
+    a.out_scores = top_scores; a.out_ids = top_ids; a.status = status;
+    EvalPackArgs pk;
+    pk.stride = trial_stride; pk.active = active; pk.n_trials = n_trials; pk.split_rows = n_active * Be;
+    cudaStream_t s = as_stream(stream);
+    dim3 grid((Be + TM - 1) / TM, a.n_splits, n_active);
+    eval_topk_f32_pack_kernel<<<grid, kEvalThreads, 0, s>>>(a, pk);
+    int rc = check_launch("hsk_eval_topk_pack");
+    if (rc) return rc;
+    // [split][trial][row] lists: one merge over the n_active * Be rows takes every trial's splits
+    if (a.n_splits > 1) rc = launch_merge_keys(a.cand, a.n_splits, n_active * Be, EV_CAP, k, top_scores, top_ids, s, nullptr, nullptr, nullptr, 0);
     return rc;
 }
 
@@ -547,4 +434,25 @@ extern "C" int hsk_rank_metrics_dense(const int32_t* top_ids, int Be, int k_max,
     a.y_true = y_true; a.n_items = n_items;
     rank_metrics_kernel<true><<<(Be + 7) / 8, 256, 0, as_stream(stream)>>>(a);
     return check_launch("hsk_rank_metrics_dense");
+}
+
+extern "C" int hsk_rank_metrics_pack(const int32_t* top_ids, int Be, int k_max, const int* ks, int n_ks, const int64_t* u_idx,
+                                     const int64_t* lab_indptr, const int32_t* lab_indices, const int32_t* user_group,
+                                     int n_groups, const float* discount, int n_trials, const int32_t* active, int n_active,
+                                     float* per_user, double* sums, int64_t* counts, int32_t* status, hsk_stream_t stream) {
+    MetricArgs a;
+    int rc = metrics_common(a, top_ids, Be, k_max, ks, n_ks, u_idx, user_group, n_groups, discount, per_user, sums, counts,
+                            "hsk_rank_metrics_pack");
+    if (rc) return rc;
+    HSK_REQUIRE(lab_indptr && lab_indices, "hsk_rank_metrics_pack: label CSR is null");
+    HSK_REQUIRE(n_trials >= 1 && n_active >= 0 && n_active <= n_trials && n_active <= 65535,
+                "hsk_rank_metrics_pack: need 0 <= n_active <= n_trials, n_trials >= 1, n_active <= 65535 (n_trials=%d n_active=%d)",
+                n_trials, n_active);
+    HSK_REQUIRE(n_active == 0 || active, "hsk_rank_metrics_pack: active is null");
+    if (Be <= 0 || n_active == 0) return HSK_OK;
+    a.lab_indptr = lab_indptr; a.lab_indices = lab_indices;
+    MetricPackArgs pk;
+    pk.active = active; pk.n_trials = n_trials; pk.groups = n_groups; pk.status = status;
+    rank_metrics_pack_kernel<<<dim3((Be + 7) / 8, n_active), 256, 0, as_stream(stream)>>>(a, pk);
+    return check_launch("hsk_rank_metrics_pack");
 }

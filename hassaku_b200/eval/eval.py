@@ -166,16 +166,8 @@ class FullEvaluator:
         if self._sums is None:
             return metrics_dict
         if self.aggr_by_group:
-            sums = self._sums.cpu().numpy()
-            counts = self._counts.cpu().numpy()
-            for g in range(-1, self.n_groups):
-                for t, k in enumerate(ks):
-                    for c, name in enumerate(METRIC_ORDER):
-                        key = name.format(k) if g == -1 else f'group_{g}_' + name.format(k)
-                        metrics_dict[key] = float(sums[g + 1, t, c]) / int(counts[g + 1])
-                    if self._hit_sums is not None:
-                        key = f'hit@{k}' if g == -1 else f'group_{g}_hit@{k}'
-                        metrics_dict[key] = float(self._hit_sums[g + 1, t]) / int(counts[g + 1])
+            metrics_dict = group_means(self._sums.cpu().numpy(), self._counts.cpu().numpy(), ks, self.n_groups,
+                                       self._hit_sums)
         else:
             per_user = torch.cat([p for p, _ in self._per_user]).cpu().numpy()
             grp = torch.cat([g for _, g in self._per_user]).cpu().numpy() if self.n_groups > 0 else None
@@ -190,6 +182,21 @@ class FullEvaluator:
                         metrics_dict[key] = (per_user[sel, t, 0] > 0).astype(per_user.dtype)
         self._reset_internal_dict()
         return metrics_dict
+
+
+def group_means(sums, counts, ks, n_groups: int, hit_sums=None) -> dict:
+    """eval.py:101-118 — {metric: mean over the users seen} from one evaluator's sums [1 + n_groups, n_ks, 3] and counts
+    [1 + n_groups] (host arrays; row 0 = all users, row 1 + g = user group g, 'group_{g}_' prefix)."""
+    metrics_dict = dict()
+    for g in range(-1, n_groups):
+        for t, k in enumerate(ks):
+            for c, name in enumerate(METRIC_ORDER):
+                key = name.format(k) if g == -1 else f'group_{g}_' + name.format(k)
+                metrics_dict[key] = float(sums[g + 1, t, c]) / int(counts[g + 1])
+            if hit_sums is not None:
+                key = f'hit@{k}' if g == -1 else f'group_{g}_hit@{k}'
+                metrics_dict[key] = float(hit_sums[g + 1, t]) / int(counts[g + 1])
+    return metrics_dict
 
 
 def accumulate_hits(hit_sums: Optional[torch.Tensor], per_user: torch.Tensor, grp: Optional[torch.Tensor],
@@ -544,3 +551,143 @@ def evaluate_recommender_algorithm(alg: RecommenderAlgorithm, eval_loader, evalu
     metrics_values = evaluator.get_results()
     log_info_results(metrics_values)
     return metrics_values
+
+
+PACK_SCRATCH_BYTES = 256 << 20   # top-k candidate scratch of one packed scoring launch (evaluate_mf_pack)
+
+
+def pack_chunk_users(batch_size: int, n_users: int, n_items: int, k: int, n_active: int,
+                     budget: int = PACK_SCRATCH_BYTES) -> int:
+    """Users per packed scoring launch: the largest multiple of the loader's batch size (up to the batches that cover
+    n_users) whose hsk_eval_topk_pack scratch for n_active trials fits `budget`, and never less than one batch."""
+    n_batches = max(1, -(-n_users // batch_size))
+    per_row = _C.eval_topk_pack_scratch_bytes(1, 1, k, 1)   # one candidate list: the scratch is at least rows x this
+    m = max(1, min(n_batches, budget // (per_row * n_active * batch_size)))
+    while m > 1 and _C.eval_topk_pack_scratch_bytes(m * batch_size, n_items, k, n_active) > budget:
+        m -= 1
+    return m * batch_size
+
+
+def _check_pack(models, evaluators):
+    """ValueError naming the condition unless `models` are SGDMatrixFactorization of one shape with fp32 evaluation and
+    `evaluators` one plain FullEvaluator per model (aggr_by_group=True, hit=False) with one K_VALUES and n_groups."""
+    shape = lambda m: (m.n_users, m.n_items, m.embedding_dim, m.use_user_bias, m.use_item_bias, m.use_global_bias)
+    if len(evaluators) != len(models):
+        raise ValueError(f'one evaluator per model: {len(models)} models, {len(evaluators)} evaluators')
+    for j, (m, ev) in enumerate(zip(models, evaluators)):
+        if not isinstance(m, SGDMatrixFactorization):
+            raise ValueError(f'model {j} is a {type(m).__name__}: packed evaluation takes SGDMatrixFactorization models')
+        if shape(m) != shape(models[0]):
+            raise ValueError(f'model {j} differs from model 0 in shape (n_users, n_items, embedding_dim, biases): '
+                             f'{shape(m)} vs {shape(models[0])}')
+        prec = getattr(m, 'eval_precision', 'fp32')
+        if prec != 'fp32':
+            raise ValueError(f"model {j} has eval_precision {prec!r}: packed evaluation runs the fp32 evaluator only")
+        if type(ev) is not FullEvaluator:
+            raise ValueError(f'evaluator {j} is a {type(ev).__name__}: packed evaluation takes plain FullEvaluator '
+                             f'objects (no calibration decorators)')
+        if not ev.aggr_by_group:
+            raise ValueError(f'evaluator {j} has aggr_by_group=False: packed evaluation returns group means only')
+        if getattr(ev, 'hit', False):
+            raise ValueError(f'evaluator {j} has hit=True: packed evaluation has no hit@k')
+        if list(ev.K_VALUES) != list(evaluators[0].K_VALUES) or ev.n_groups != evaluators[0].n_groups:
+            raise ValueError(f'evaluator {j} differs from evaluator 0 in K_VALUES or n_groups')
+
+
+def _pack_trials(models):
+    """(flat [n_trials, stride] view of the allocation, trial index per model) for models whose arenas are rows of one
+    [M, stride] CUDA allocation, as PackedMFTrainStep binds them; ValueError naming the condition otherwise."""
+    stride = models[0].layout.n_total
+    storage = models[0].arena.untyped_storage().data_ptr()
+    idx = []
+    for j, m in enumerate(models):
+        a = m.arena
+        if (not a.is_cuda or a.dtype != torch.float32 or a.dim() != 1 or a.numel() != stride or a.stride(0) != 1
+                or a.untyped_storage().data_ptr() != storage or a.storage_offset() % stride != 0):
+            raise ValueError(f'model {j} arena is not a row of the [M, {stride}] CUDA allocation of model 0: packed '
+                             f'evaluation needs the models bound as PackedMFTrainStep binds them')
+        idx.append(a.storage_offset() // stride)
+    if len(set(idx)) != len(idx):
+        raise ValueError('two models share one row of the allocation')
+    flat = models[0].arena.detach().as_strided((max(idx) + 1, stride), (stride, 1), 0)
+    return flat, idx
+
+
+def evaluate_mf_pack(models, eval_loader, evaluators, device='cpu', verbose=False) -> list:
+    """`[evaluate_recommender_algorithm(models[j], eval_loader, evaluators[j], device, verbose) for j]` in one packed
+    sweep: per chunk of users one hsk_eval_topk_pack and one hsk_rank_metrics_pack launch for all the models, and one
+    device-to-host copy for the whole sweep.  `models`: SGDMatrixFactorization of one shape whose arenas are rows of one
+    [M, stride] allocation (PackedMFTrainStep binds them so; any subset, any order), fp32 evaluation; `evaluators`: plain
+    FullEvaluator with aggr_by_group=True and hit=False, one per model, sharing K_VALUES and the user groups.  Anything
+    else raises ValueError.
+
+    A chunk is the largest multiple of the loader's batch size whose scratch fits PACK_SCRATCH_BYTES: a user's top-k
+    list depends on that user's row alone, so the chunk does not change the ids.  Under torch.use_deterministic_algorithms
+    the metric sums are taken per loader batch in order (hsk_rank_metrics_sums_det_pack), bitwise as the per-model path."""
+    models, evaluators = list(models), list(evaluators)
+    if not models:
+        return []
+    _check_pack(models, evaluators)
+    flat, idx = _pack_trials(models)
+    ev0, alg0 = evaluators[0], models[0]
+    if alg0.n_items < max(ev0.K_VALUES):
+        raise RuntimeError('selected index k out of range')  # as evaluate_mf_sweep
+    dev = flat.device
+    dataset = eval_loader.dataset
+    labels = device_csr(dataset, 'iteration_matrix', dev)
+    exclude = device_csr(dataset, 'exclude_data', dev)
+    for ev in evaluators:
+        ev._prepare(dev)
+    G, ks = ev0.n_groups, ev0._ks()
+    group = ev0._group_dev
+    for j, ev in enumerate(evaluators[1:], 1):
+        if G > 0 and not torch.equal(ev._group_dev, group):
+            raise ValueError(f'evaluator {j} differs from evaluator 0 in user_to_user_group')
+    M, T, n_ks, k = len(models), flat.shape[0], len(ks), ks[0]
+    n_users = dataset.n_users
+    bs = getattr(eval_loader, 'batch_size', None) or 8192
+    chunk = pack_chunk_users(bs, n_users, alg0.n_items, k, M, PACK_SCRATCH_BYTES)
+    # sums [T, 1 + G, n_ks, 3] fp64, counts [T, 1 + G] int64 and the status word in one buffer: one copy reads them all
+    n_sums, n_counts = T * (1 + G) * n_ks * 3, T * (1 + G)
+    acc = torch.zeros(n_sums + n_counts + 1, dtype=torch.float64, device=dev)
+    sums = acc[:n_sums].view(T, 1 + G, n_ks, 3)
+    counts = acc[n_sums:n_sums + n_counts].view(torch.int64).view(T, 1 + G)
+    status = acc[n_sums + n_counts:].view(torch.int32)[:1]
+    for j, ev in zip(idx, evaluators):        # what the evaluators already hold, as the per-model sweep would add to it
+        sums[j].copy_(ev._sums)
+        counts[j].copy_(ev._counts)
+    det = determinism.enabled()
+    metric_sums = torch.zeros_like(sums) if det else sums
+    active = torch.tensor(idx, dtype=torch.int32).to(dev)
+    Bc = min(chunk, n_users)
+    scratch = torch.empty(_C.eval_topk_pack_scratch_bytes(Bc, alg0.n_items, k, M), dtype=torch.uint8, device=dev)
+    top_s = torch.empty(M * Bc * k, dtype=torch.float32, device=dev)
+    top_i = torch.empty(M * Bc * k, dtype=torch.int32, device=dev)
+    per_user = torch.empty(M * Bc * n_ks * 3, dtype=torch.float32, device=dev) if det else None
+    discount = discount_table(k, dev)
+    tables = alg0.layout.tables(flat[0])
+    starts = range(0, n_users, chunk)
+    with torch.no_grad(), nvtx.range('hsk.eval_pack_sweep'):
+        for s in (tqdm(starts) if verbose else starts):
+            u = torch.arange(s, min(s + chunk, n_users), dtype=torch.int64, device=dev)
+            Be = u.numel()
+            ids = top_i[:M * Be * k].view(M, Be, k)
+            _C.eval_topk_pack(tables, flat.shape[1], T, active, u, k, top_s[:M * Be * k].view(M, Be, k), ids, scratch,
+                              exclude.indptr, exclude.indices, status=status)
+            pu = per_user[:M * Be * n_ks * 3].view(M, Be, n_ks, 3) if det else None
+            _C.rank_metrics_pack(ids, ks, u, labels.indptr, labels.indices, discount, active, metric_sums, counts,
+                                 user_group=group, n_groups=G, per_user=pu, status=status)
+            if det:
+                _C.rank_metrics_sums_det_pack(pu, u, bs, active, sums, user_group=group, n_groups=G, status=status)
+    host = acc.cpu()
+    if int(host[n_sums + n_counts:].view(torch.int32)[0]) & _C.STATUS_BAD_INDEX:
+        raise IndexError('index out of range in SGDMatrixFactorization (user or item index)')
+    host_sums = host[:n_sums].view(T, 1 + G, n_ks, 3).numpy()
+    host_counts = host[n_sums:n_sums + n_counts].view(torch.int64).view(T, 1 + G).numpy()
+    out = []
+    for j, ev in zip(idx, evaluators):
+        ev._reset_internal_dict()
+        metrics_values = group_means(host_sums[j], host_counts[j], ks, G)
+        log_info_results(metrics_values)
+        out.append(metrics_values)
+    return out

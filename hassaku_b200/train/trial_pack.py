@@ -20,6 +20,9 @@ that stop early simply stop consuming them.
 `PackedTrainer` is `Trainer.fit` for the M trials over one shared loader: per trial the initial validation, early stopping
 on its own `optimizing_metric` / `max_patience` / `n_epochs`, a checkpoint to its `model_path` on every improvement, the
 same prints and the same returned dict.  A trial that runs out of patience or epochs is deactivated at that epoch boundary.
+The initial validation and each epoch's validation are one packed sweep over the trials concerned (evaluate_mf_pack:
+one top-k and one metrics launch per chunk of users for all of them); models with a tensor-core `eval_precision` are
+validated one by one instead.
 
 Packing pays where one trial's step is launch-bound (measured on a B200 at the ML-1M shape: up to 11.6x at B 64, d 64;
 2.1x at d 402, where the pack's AdamW pass runs at HBM bandwidth).  It does not pay for bpr / bce with d > 96 at large
@@ -35,7 +38,7 @@ import torch
 
 from hassaku_b200 import _C, determinism
 from hassaku_b200.algorithms.sgd_alg import SGDMatrixFactorization
-from hassaku_b200.eval.eval import FullEvaluator, evaluate_recommender_algorithm
+from hassaku_b200.eval.eval import FullEvaluator, evaluate_mf_pack, evaluate_recommender_algorithm
 from hassaku_b200.train.optim import stamp_segments
 from hassaku_b200.train.rec_losses import RecommenderSystemLoss
 from hassaku_b200.train.trainer_step import HostBatchStager
@@ -311,15 +314,36 @@ class PackedTrainer:
         self.schedule = TrialSchedule([c['n_epochs'] for c in confs], [c['max_patience'] for c in confs])
         self.epoch_losses = [[] for _ in confs]    # per trial, the dicts of its train epochs
 
+    def _evaluator(self) -> FullEvaluator:
+        ds = self.val_loader.dataset
+        return FullEvaluator(aggr_by_group=True, n_groups=ds.n_user_groups, user_to_user_group=ds.user_to_user_group)
+
     @torch.no_grad()
     def val(self, j: int) -> dict:
         """Trainer.val for trial j: full-rank evaluation on the validation loader -> metric dict."""
         model = self.models[j]
         model.eval()
         print('Validation started')
-        ds = self.val_loader.dataset
-        evaluator = FullEvaluator(aggr_by_group=True, n_groups=ds.n_user_groups, user_to_user_group=ds.user_to_user_group)
-        return evaluate_recommender_algorithm(model, self.val_loader, evaluator, self.device, self.batch_verbose)
+        return evaluate_recommender_algorithm(model, self.val_loader, self._evaluator(), self.device, self.batch_verbose)
+
+    @torch.no_grad()
+    def val_pack(self, trials) -> dict:
+        """Trainer.val for every trial of `trials` in one packed sweep -> {trial: metric dict}; {} when a model evaluates
+        in a tensor-core precision (evaluate_mf_pack runs the fp32 evaluator only: such packs use `val` per trial)."""
+        if any(getattr(m, 'eval_precision', 'fp32') != 'fp32' for m in self.models):
+            return {}
+        for j in trials:
+            self.models[j].eval()
+        res = evaluate_mf_pack([self.models[j] for j in trials], self.val_loader, [self._evaluator() for _ in trials],
+                               self.device, self.batch_verbose)
+        return dict(zip(trials, res))
+
+    def _val_result(self, j: int, packed: dict) -> dict:
+        """Trial j's validation: its entry of the packed sweep (with val's print), or `val(j)`."""
+        if j not in packed:
+            return self.val(j)
+        print('Validation started')
+        return packed[j]
 
     def _train_one_epoch(self, active) -> dict:
         for j in active:
@@ -337,8 +361,9 @@ class PackedTrainer:
 
     def fit(self):
         sch = self.schedule
+        packed = self.val_pack(list(range(len(self.confs))))
         for j, conf in enumerate(self.confs):
-            first = self.val(j)
+            first = self._val_result(j, packed)
             sch.start(j, first[conf['optimizing_metric']], first)
             print('Init - Avg Val Value {:.3f} \n'.format(sch.best_value[j]))
             self.models[j].save_model_to_path(conf['model_path'])
@@ -351,13 +376,14 @@ class PackedTrainer:
             self.train_step.set_active([j in active for j in range(len(self.confs))])
             self.train_step.prepare(len(self.train_loader))
             losses = self._train_one_epoch(active)
+            packed = self.val_pack(active)
             epoch = sch.epoch
             for j in active:
                 lj = losses[j]
                 self.epoch_losses[j].append(lj)
                 print('Epoch {} - Epoch Avg Train Loss {:.4f} ({:.4f} Rec Loss + {:.4f} Reg Loss )\n'.format(
                     epoch, lj['epoch_train_loss'], lj['epoch_train_rec_loss'], lj['epoch_train_reg_loss']))
-                metrics = self.val(j)
+                metrics = self._val_result(j, packed)
                 value = metrics[self.confs[j]['optimizing_metric']]
                 print('Epoch {} - Avg Val Value {:.4f} \n'.format(epoch, value))
                 if sch.end_epoch(j, value, metrics):

@@ -431,6 +431,36 @@ HSK_API int hsk_adamw_consts_table(const double* lr /* host [n_trials] */, const
                                    int n_trials, double beta1, double beta2, double eps, int64_t first_step, int n_steps,
                                    float* out /* host [n_steps, n_trials, 8] */);
 
+/* ---- packed validation: the fp32 evaluator and its metrics for every active trial of a pack in one launch each ---------
+ * Same layout and `active` rules as above (an out-of-range entry sets HSK_STATUS_BAD_INDEX and its CTAs write nothing;
+ * its output rows are then undefined).  Single GPU: no id mapping, u_rows or item shards.
+ *   hsk_eval_topk_pack  hsk_eval_topk (fp32, id_offset 0, id_stride 1) of every active trial on ONE shared user batch
+ *       u_idx [Be] and ONE shared exclusion CSR: top_scores / top_ids [n_active, Be, k], row a * Be + r = trial active[a],
+ *       user u_idx[r].  Each row is bitwise what hsk_eval_topk returns for that trial and user, whatever Be and n_active
+ *       (a row's per-item arithmetic and key order do not depend on the launch shape).  The item split plan counts
+ *       n_active times the row tiles, so items are not split where the trials already fill the GPU; scratch:
+ *       hsk_eval_topk_pack_scratch_bytes(Be, t->n_items, k, n_active) bytes.  n_active * Be < 2^31.
+ *   hsk_rank_metrics_pack  hsk_rank_metrics (CSR labels) of top_ids [n_active, Be, k_max]: trial active[a] adds into its
+ *       own slices sums [n_trials, 1 + n_groups, n_ks, 3] (fp64) and counts [n_trials, 1 + n_groups]; per_user (nullable)
+ *       [n_active, Be, n_ks, 3].
+ *   hsk_rank_metrics_sums_det_pack  hsk_rank_metrics_sums_det for per_user [n_active, Be, n_ks, 3] into the same sums
+ *       layout: each trial's Be rows are cut into consecutive batches of `batch` rows (the last may be shorter) and
+ *       added batch by batch, in order — bitwise what one hsk_rank_metrics_sums_det call per batch gives. */
+HSK_API int64_t hsk_eval_topk_pack_scratch_bytes(int Be, int64_t n_items, int k, int n_active);
+HSK_API int hsk_eval_topk_pack(const hsk_mf_tables* t, int64_t trial_stride, int n_trials, const int32_t* active, int n_active,
+                               const int64_t* u_idx, int Be, const int64_t* excl_indptr /* [n_users + 1] or NULL */,
+                               const int32_t* excl_indices, int k /* <= 128 */, float* top_scores, int32_t* top_ids,
+                               void* scratch, int64_t scratch_bytes, int32_t* status, hsk_stream_t stream);
+HSK_API int hsk_rank_metrics_pack(const int32_t* top_ids, int Be, int k_max, const int* ks /* host */, int n_ks,
+                                  const int64_t* u_idx, const int64_t* lab_indptr, const int32_t* lab_indices,
+                                  const int32_t* user_group /* [n_users] or NULL */, int n_groups, const float* discount,
+                                  int n_trials, const int32_t* active, int n_active, float* per_user /* nullable */,
+                                  double* sums, int64_t* counts, int32_t* status, hsk_stream_t stream);
+HSK_API int hsk_rank_metrics_sums_det_pack(const float* per_user, int Be, int batch, int n_ks, const int64_t* u_idx,
+                                           const int32_t* user_group /* nullable */, int n_groups, int n_trials,
+                                           const int32_t* active, int n_active, double* sums, int32_t* status,
+                                           hsk_stream_t stream);
+
 /* ==== deterministic mode (hsk_det.cu): bitwise-reproducible training / evaluation reductions ========================
  * What the Python layer runs under torch.use_deterministic_algorithms(True).  The batch is grouped by row (stable radix
  * sort of the item ids of the B * N1 slots and of the user ids of the B samples) and every touched row is produced by ONE
