@@ -238,7 +238,8 @@ HSK_API int hsk_adamw_dense(float* p, float* m, float* v, float* g, int64_t n, d
  * segments whose stamp byte differs from this step's stamp g is neither read nor re-zeroed: 24 B / element instead of
  * 32 B.  Contract: g is all-zero outside the rows stamped this step — hsk_adamw_dense_rows leaves it so, and every
  * caller that scatters gradients into rows calls hsk_mark_rows on their indices with the same step.  Everything
- * outside the segments (bias vectors, padding) takes the plain dense path.  The stamp of step t is hsk_row_stamp(t) =
+ * outside the segments (bias vectors, padding) takes the plain dense path, in the same launch: one kernel per call.
+ * The stamp of step t is hsk_row_stamp(t) =
  * 1 + t % 255: the stamp arrays are never cleared (start them at 0).
  * Graph mode (both non-null): consts_dev = the 8 fp32 of hsk_adamw_consts for the step, step_dev = the 1-based step
  * count in device memory (it selects the stamp), so that one captured launch serves every step; lr ... step are then
