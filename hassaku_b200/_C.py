@@ -91,6 +91,10 @@ def _declare(lib):
         'hsk_mark_rows': (i32, [vp, i64, i64, vp, i64, vp, vp]),
         'hsk_mark_batch': (i32, [vp, vp, i32, i32, i64, i64, vp, vp, i64, vp, vp]),
         'hsk_adamw_dense_rows': (i32, [vp, vp, vp, vp, i64, C.POINTER(RowSegment), i32, f64, f64, f64, f64, f64, i64, vp, vp, i32, i32, vp]),
+        'hsk_adamw_dense_rows_lag': (i32, [vp, vp, vp, vp, i64, C.POINTER(RowSegment), i32, C.POINTER(vp), C.POINTER(vp), i32,
+                                           f64, f64, f64, f64, f64, i64, i32, i32, vp]),
+        'hsk_adamw_lag_sync': (i32, [vp, vp, i64, C.POINTER(RowSegment), i32, C.POINTER(vp), C.POINTER(vp), f64, f64, i64, i32,
+                                     vp]),
         'hsk_rescore_topk': (i32, [T, vp, i32, i64, i64, vp, vp, i32, i32, vp, vp, vp, vp]),
         'hsk_rescore_scores': (i32, [T, vp, i32, i64, i64, vp, i32, vp, vp, vp]),
         'hsk_topk_combine': (i32, [vp, vp, vp, i32, i32, i32, i32, vp, vp, vp]),
@@ -458,6 +462,46 @@ def adamw_dense_rows(p, m, v, g, segments, lr, beta1, beta2, eps, weight_decay, 
         _check(lib().hsk_adamw_dense_rows(p.data_ptr(), m.data_ptr(), v.data_ptr(), g.data_ptr(), p.numel(), arr, len(segs),
                                           lr, beta1, beta2, eps, weight_decay, step, _ptr(consts_dev), _ptr(step_dev), arith,
                                           int(adam_l2), st), 'hsk_adamw_dense_rows')
+
+
+def adamw_dense_rows_lag(p, m, v, g, segments, bases, lag: int, lr, beta1, beta2, eps, weight_decay, step: int,
+                         arith: int = 0, adam_l2: bool = False):
+    """adamw_dense_rows with the segments' m and v written back once every `lag` steps (hsk_adamw_dense_rows_lag).
+    bases: per segment (base_in, base_out), two [n_rows] uint8 tensors; swap them after the call."""
+    for n, t in (('p', p), ('m', m), ('v', v), ('g', g)):
+        _req(t, torch.float32, n)
+    segs, arr = _row_segments(segments, 'adamw_dense_rows_lag')
+    b_in, b_out = _lag_bases(segs, bases, 'adamw_dense_rows_lag')
+    with _on_device_of(p, m, v, g, *[sg[3] for sg in segs], *[b for pair in bases for b in pair]) as st:
+        _check(lib().hsk_adamw_dense_rows_lag(p.data_ptr(), m.data_ptr(), v.data_ptr(), g.data_ptr(), p.numel(), arr,
+                                              len(segs), b_in, b_out, lag, lr, beta1, beta2, eps, weight_decay, step, arith,
+                                              int(adam_l2), st), 'hsk_adamw_dense_rows_lag')
+
+
+def adamw_lag_sync(m, v, segments, bases, beta1, beta2, step: int, arith: int = 0):
+    """every row of the segments to step `step` (hsk_adamw_lag_sync); swap the bases after the call"""
+    for n, t in (('m', m), ('v', v)):
+        _req(t, torch.float32, n)
+    if m.numel() != v.numel():
+        raise HskError('adamw_lag_sync: m and v must have the same number of elements')
+    segs, arr = _row_segments(segments, 'adamw_lag_sync')
+    b_in, b_out = _lag_bases(segs, bases, 'adamw_lag_sync')
+    with _on_device_of(m, v, *[b for pair in bases for b in pair]) as st:
+        _check(lib().hsk_adamw_lag_sync(m.data_ptr(), v.data_ptr(), m.numel(), arr, len(segs), b_in, b_out, beta1, beta2,
+                                        step, arith, st), 'hsk_adamw_lag_sync')
+
+
+def _lag_bases(segs, bases, who):
+    bases = list(bases)
+    if len(bases) != len(segs):
+        raise HskError(f'{who}: one (base_in, base_out) pair per segment')
+    b_in, b_out = (C.c_void_p * max(len(segs), 1))(), (C.c_void_p * max(len(segs), 1))()
+    for k, ((_off, rows, _ld, _st), (bi, bo)) in enumerate(zip(segs, bases)):
+        _req(bi, torch.uint8, 'base_in'); _req(bo, torch.uint8, 'base_out')
+        if bi.numel() < rows or bo.numel() < rows:
+            raise HskError(f'{who}: base array shorter than the segment')
+        b_in[k], b_out[k] = bi.data_ptr(), bo.data_ptr()
+    return b_in, b_out
 
 
 def _row_segments(segments, who):

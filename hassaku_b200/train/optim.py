@@ -3,10 +3,15 @@
 every step, zero-gradient rows included (SURVEY A.5), and the gradient arena is zeroed in the same pass (replaces
 optimizer.zero_grad()).  When a batch touches a small part of a table (cfg4: 0.35 M of 3 M rows) the rows kernel skips
 the gradient READ and re-zeroing of the untouched rows — their gradient is exactly zero, so the result is bit-identical
-to the plain dense kernel at 24 instead of 32 bytes per parameter."""
+to the plain dense kernel at 24 instead of 32 bytes per parameter.  With `state_lag` K > 1 (AdamW, or Adam without
+weight decay) those rows also write m and v back only once every K steps (hsk_adamw_dense_rows_lag): 16 + 8 / K bytes per
+parameter.  p is current after every step, and `m` / `v` bring every row up to date before they are returned."""
 import torch
 
 from hassaku_b200 import _C
+
+# m / v write-back period of untouched rows (DenseAdam state_lag), measured at cfg4: profiles/adamw_lag_cost.json
+DEFAULT_STATE_LAG = 8
 
 
 def stamp_segments(lay, B: int, n_slots: int, stamp_users, stamp_items):
@@ -29,7 +34,9 @@ class DenseAdam(torch.optim.Optimizer):
     (the reference always passes conf['wd'])."""
 
     def __init__(self, model, lr: float = 1e-3, weight_decay: float = 0.0, betas=(0.9, 0.999), eps: float = 1e-8,
-                 decoupled: bool = True, arith: int = 0, mode: str = 'dense'):
+                 decoupled: bool = True, arith: int = 0, mode: str = 'dense', state_lag: int = DEFAULT_STATE_LAG):
+        if not 1 <= int(state_lag) <= 128:
+            raise ValueError('state_lag must be in [1, 128]')
         self.model = model
         super().__init__(list(model.parameters()),
                          dict(lr=lr, weight_decay=weight_decay, betas=betas, eps=eps, decoupled=decoupled))
@@ -39,16 +46,20 @@ class DenseAdam(torch.optim.Optimizer):
         if mode == 'lazy' and not decoupled:
             raise ValueError('lazy mode is defined for AdamW (decoupled decay) only')
         self.mode = mode
-        self.t = 0
+        self.state_lag = int(state_lag) if mode == 'dense' else 1
+        self._t = 0
         self._segments = ()      # row segments whose untouched rows skip the gradient traffic in the NEXT step_fused
+        self._behind = {}        # segment offset -> segment: tables whose rows' m / v may be older than step t
+        self._lag_key = None     # (beta1, beta2, arith, lag) the rows of _behind were stepped with
+        self._base_t = {}        # segment offset -> the step that base_in holds for every row of the table
         self._alloc()
 
     def _alloc(self):
         arena = self.model.arena
         if not arena.is_cuda:
             raise _C.HskError('DenseAdam needs the model on a CUDA device (no CPU path)')
-        self.m = torch.zeros_like(arena)
-        self.v = torch.zeros_like(arena)
+        self._m = torch.zeros_like(arena)
+        self._v = torch.zeros_like(arena)
         self.g = torch.zeros_like(arena)
         self.grad_tables = self.model.layout.tables(self.g)
         lay = self.model.layout
@@ -58,6 +69,46 @@ class DenseAdam(torch.optim.Optimizer):
         else:   # per-row step stamps (hsk_row_stamp): never cleared
             self.stamp_users = torch.zeros(lay.n_users, dtype=torch.uint8, device=arena.device)
             self.stamp_items = torch.zeros(lay.n_items, dtype=torch.uint8, device=arena.device)
+            if self.state_lag > 1:   # per row the step & 255 of its last m / v write-back: [base_in, base_out]
+                self._bases = {off: [torch.zeros(rows, dtype=torch.uint8, device=arena.device) for _ in range(2)]
+                               for off, rows in ((lay.off_U, lay.n_users), (lay.off_V, lay.n_items))}
+
+    @property
+    def t(self):
+        return self._t
+
+    @t.setter
+    def t(self, step: int):
+        self.sync_state()
+        self._t = int(step)
+
+    @property
+    def m(self):
+        """first moments of the arena, every row current"""
+        self.sync_state()
+        return self._m
+
+    @property
+    def v(self):
+        """second moments of the arena, every row current"""
+        self.sync_state()
+        return self._v
+
+    def sync_state(self):
+        """Bring the m and v of every row to step t (rows the last steps did not write back are behind)."""
+        if not self._behind:
+            return
+        segs = tuple(self._behind.values())
+        b1, b2, arith, _ = self._lag_key
+        _C.adamw_lag_sync(self._m, self._v, segs, [self._bases[sg[0]] for sg in segs], b1, b2, self._t, arith=arith)
+        for sg in segs:
+            self._swap_bases(sg[0])
+        self._behind = {}
+
+    def _swap_bases(self, off):
+        b = self._bases[off]
+        b[0], b[1] = b[1], b[0]
+        self._base_t[off] = self._t
 
     @property
     def grad_views(self):
@@ -74,7 +125,7 @@ class DenseAdam(torch.optim.Optimizer):
             return
         segs, su, si = stamp_segments(lay, int(u_idxs.numel()), int(i_idxs.numel()), self.stamp_users, self.stamp_items)
         if segs:
-            _C.mark_batch(u_idxs, i_idxs, lay.n_users, lay.n_items, su, si, step=self.t + 1)
+            _C.mark_batch(u_idxs, i_idxs, lay.n_users, lay.n_items, su, si, step=self._t + 1)
         self._segments = segs
 
     def _step_lazy(self, grp):
@@ -90,29 +141,47 @@ class DenseAdam(torch.optim.Optimizer):
                                             (lay.off_V, lay.off_Ib, lay.n_items, self.touched_items)):
             bias = None
             if off_b >= 0:
-                bias = tuple(vec(a, off_b, rows) for a in (arena, self.m, self.v, self.g))
-            _C.adamw_rows_lazy(t2d(arena, off_t, rows), t2d(self.m, off_t, rows), t2d(self.v, off_t, rows),
+                bias = tuple(vec(a, off_b, rows) for a in (arena, self._m, self._v, self.g))
+            _C.adamw_rows_lazy(t2d(arena, off_t, rows), t2d(self._m, off_t, rows), t2d(self._v, off_t, rows),
                                t2d(self.g, off_t, rows), touched, grp['lr'], grp['betas'][0], grp['betas'][1], grp['eps'],
-                               grp['weight_decay'], self.t, bias=bias)
+                               grp['weight_decay'], self._t, bias=bias)
         if lay.off_Gb >= 0:   # the global bias is touched by every sample: plain dense update of that one element
             sl = slice(lay.off_Gb, lay.off_Gb + 4)
-            _C.adamw_dense(arena[sl], self.m[sl], self.v[sl], self.g[sl], grp['lr'], grp['betas'][0], grp['betas'][1],
-                           grp['eps'], grp['weight_decay'], self.t, arith=self.arith, zero_grad=True)
+            _C.adamw_dense(arena[sl], self._m[sl], self._v[sl], self.g[sl], grp['lr'], grp['betas'][0], grp['betas'][1],
+                           grp['eps'], grp['weight_decay'], self._t, arith=self.arith, zero_grad=True)
 
     def step_fused(self):
         """One optimizer step consuming the gradient arena `self.g` (filled by hsk_mf_train_fused)."""
         grp = self.param_groups[0]
-        self.t += 1
         if self.mode == 'lazy':
+            self._t += 1
             return self._step_lazy(grp)
         segs, self._segments = self._segments, ()
-        if segs:
-            _C.adamw_dense_rows(self.model.arena, self.m, self.v, self.g, segs, grp['lr'], grp['betas'][0], grp['betas'][1],
-                                grp['eps'], grp['weight_decay'], self.t, arith=self.arith, adam_l2=not grp['decoupled'])
+        b1, b2 = grp['betas']
+        key = (b1, b2, self.arith, self.state_lag)
+        lag = self.state_lag > 1 and bool(segs) and (grp['decoupled'] or grp['weight_decay'] == 0.0)
+        offs = {sg[0] for sg in segs}
+        if self._behind and not (lag and key == self._lag_key and self._behind.keys() <= offs):
+            self.sync_state()    # the rows behind are brought up to date with what they were stepped with
+        self._t += 1
+        p, m, v, g = self.model.arena, self._m, self._v, self.g
+        if lag:
+            for off in offs:     # a table entering the lagged update: every row's m / v are those of step t - 1
+                if self._base_t.get(off) != self._t - 1:
+                    self._bases[off][0].fill_((self._t - 1) & 255)
+            _C.adamw_dense_rows_lag(p, m, v, g, segs, [self._bases[sg[0]] for sg in segs], self.state_lag, grp['lr'], b1,
+                                    b2, grp['eps'], grp['weight_decay'], self._t, arith=self.arith,
+                                    adam_l2=not grp['decoupled'])
+            for sg in segs:
+                self._swap_bases(sg[0])
+                self._behind[sg[0]] = sg
+            self._lag_key = key
+        elif segs:
+            _C.adamw_dense_rows(p, m, v, g, segs, grp['lr'], b1, b2, grp['eps'], grp['weight_decay'], self._t,
+                                arith=self.arith, adam_l2=not grp['decoupled'])
         else:
-            _C.adamw_dense(self.model.arena, self.m, self.v, self.g, grp['lr'], grp['betas'][0], grp['betas'][1],
-                           grp['eps'], grp['weight_decay'], self.t, arith=self.arith, adam_l2=not grp['decoupled'],
-                           zero_grad=True)
+            _C.adamw_dense(p, m, v, g, grp['lr'], b1, b2, grp['eps'], grp['weight_decay'], self._t, arith=self.arith,
+                           adam_l2=not grp['decoupled'], zero_grad=True)
 
     @torch.no_grad()
     def step(self, closure=None):

@@ -262,6 +262,31 @@ HSK_API int hsk_adamw_dense_rows(float* p, float* m, float* v, float* g, int64_t
                                  double weight_decay, int64_t step, const float* consts_dev, const int64_t* step_dev,
                                  int arith, int adam_l2, hsk_stream_t stream);
 
+/* ---- hsk_adamw_dense_rows with the moments of untouched rows written back once every `lag` steps ---------------------
+ * p after every call, and m and v after hsk_adamw_lag_sync, are bit for bit those of hsk_adamw_dense_rows with the same
+ * arguments.  A row of a segment keeps the m and v of the step `base` at which they were last written; a call replays
+ * the steps without gradient since then in registers (m and v of such a step depend on beta1, beta2 and the old values
+ * only), applies step `step`, stores p, and writes m and v back (base = step) only when the row is stamped this step or
+ * (step + row) % lag == 0 — else 16 instead of 24 bytes per parameter.  Everything outside the segments is updated as in
+ * hsk_adamw_dense_rows.  lag = 1 writes every row every step: hsk_adamw_dense_rows exactly.
+ * base_in[s] / base_out[s] (host arrays of n_segments device pointers; for every non-empty segment two distinct
+ * [n_rows] byte arrays): base & 255 per row is read from base_in and written to base_out for every row; the caller
+ * swaps them after the call.  Contract: 1 <= step - base <= lag for every row — start a segment with base = step - 1 of
+ * its first call (its m and v current), call with consecutive steps, and sync before any other update of m and v, a
+ * change of beta1 / beta2 / arith / lag, or a read of m and v.  Only AdamW (decoupled decay) or Adam with
+ * weight_decay = 0: L2 decay gives untouched rows a non-zero gradient.  No graph mode (consts_dev / step_dev). */
+HSK_API int hsk_adamw_dense_rows_lag(float* p, float* m, float* v, float* g, int64_t n,
+                                     const hsk_row_segment* segments /* host */, int n_segments /* <= 4 */,
+                                     const uint8_t* const* base_in /* host */, uint8_t* const* base_out /* host */,
+                                     int lag /* 1..128 */, double lr, double beta1, double beta2, double eps,
+                                     double weight_decay, int64_t step, int arith, int adam_l2, hsk_stream_t stream);
+/* every row of the segments to step `step` (the last step taken): replays its steps without gradient since base_in,
+ * writes m and v, and sets base_out = step for every row (swap after the call).  The segments' stamps are not read. */
+HSK_API int hsk_adamw_lag_sync(float* m, float* v, int64_t n, const hsk_row_segment* segments /* host */,
+                               int n_segments /* <= 4 */, const uint8_t* const* base_in /* host */,
+                               uint8_t* const* base_out /* host */, double beta1, double beta2, int64_t step, int arith,
+                               hsk_stream_t stream);
+
 /* ---- a10: uniform negative sampling on the device (data/dataloader.py:56-57, 92-129) -------------------------------
  * For every batch row b: i_idx[b, 0] = pos_idx[b] (if pos_idx != NULL) and i_idx[b, 1..N] = N items drawn uniformly
  * from [0, n_items) none of which is a TRAIN item of user u_idx[b] (CSR of the training interactions: indptr int64
