@@ -214,7 +214,7 @@ extern "C" int64_t hsk_route_scratch_bytes(int64_t n_items, int G) {
 extern "C" int hsk_route_items(const int64_t* i_idx, int64_t n, int64_t n_items, int G, int capq, int ld, int32_t* req_rows,
                                int32_t* req_count, int64_t* compact_idx, void* scratch, int64_t scratch_bytes,
                                int32_t* status, hsk_stream_t stream) {
-    HSK_REQUIRE(i_idx && req_rows && req_count && compact_idx && scratch, "hsk_route_items: null pointer");
+    HSK_REQUIRE(req_rows && req_count && scratch && (n == 0 || (i_idx && compact_idx)), "hsk_route_items: null pointer");
     HSK_REQUIRE(n >= 0 && n_items >= 1 && G >= 1 && capq >= 1 && ld >= 4 && ld % 4 == 0, "hsk_route_items: bad sizes");
     HSK_REQUIRE(scratch_bytes >= hsk_route_scratch_bytes(n_items, G), "hsk_route_items: scratch too small");
     HSK_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 15) == 0, "hsk_route_items: scratch must be 16-byte aligned");

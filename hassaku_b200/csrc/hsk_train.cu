@@ -193,7 +193,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32) mf_train_fused_pack_kernel(
 static int fill_args(TrainArgs& a, const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx,
                      const int64_t* i_idx, int B, int N1, const char* who) {
     HSK_REQUIRE(t && t->Uw && t->Vw, "%s: tables are null", who);
-    HSK_REQUIRE(u_idx && i_idx, "%s: index pointers are null", who);
+    HSK_REQUIRE(B == 0 || (u_idx && i_idx), "%s: index pointers are null", who);   // an empty batch may come as null
     HSK_REQUIRE(B >= 0 && N1 >= 1, "%s: need B >= 0 and N1 >= 1 (B=%d N1=%d)", who, B, N1);
     HSK_REQUIRE(t->d >= 1 && t->ld >= t->d && (t->ld % 4) == 0, "%s: need 1 <= d <= ld and ld %% 4 == 0 (d=%d ld=%d)", who,
                 t->d, t->ld);
@@ -302,7 +302,7 @@ extern "C" int hsk_mf_train_fused_peer(const hsk_mf_tables* t, const hsk_mf_tabl
                                        const int64_t* u_idx, const int64_t* i_idx, int B, int N1, int64_t B_global,
                                        int loss_kind, float neg_shift, double* loss_accum, int64_t step,
                                        const int64_t* step_dev, int32_t* status, hsk_stream_t stream) {
-    HSK_REQUIRE(t && g && peers && t->Uw && g->Uw && u_idx && i_idx, "hsk_mf_train_fused_peer: null pointer");
+    HSK_REQUIRE(t && g && peers && t->Uw && g->Uw && (B == 0 || (u_idx && i_idx)), "hsk_mf_train_fused_peer: null pointer");
     HSK_REQUIRE(peers->world >= 1 && peers->world <= HSK_MAX_PEERS, "hsk_mf_train_fused_peer: world must be 1..%d", HSK_MAX_PEERS);
     HSK_REQUIRE(B >= 0 && N1 >= 1 && B_global >= B, "hsk_mf_train_fused_peer: bad batch sizes (B=%d N1=%d)", B, N1);
     HSK_REQUIRE(t->d >= 1 && t->ld >= t->d && (t->ld % 4) == 0 && g->ld == t->ld, "hsk_mf_train_fused_peer: bad row layout");

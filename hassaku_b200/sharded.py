@@ -115,6 +115,10 @@ class ShardedMF:
                  world: Optional[int] = None, rank: Optional[int] = None, device='cuda', ops=None, group=None):
         world = dist.get_world_size(group) if world is None else world
         rank = dist.get_rank(group) if rank is None else rank
+        if n_users < world or n_items < world:
+            # a rank without a user or an item row would hand the kernels empty tables
+            raise ValueError(f'ShardedMF needs at least one user row and one item row per rank: n_users ({n_users}) and '
+                             f'n_items ({n_items}) must be >= world ({world})')
         self.spec = ShardSpec(world, rank, n_users, n_items)
         self.d, self.group, self.device = d, group, torch.device(device)
         self.flags = (use_user_bias, use_item_bias, use_global_bias)

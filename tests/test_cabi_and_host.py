@@ -243,3 +243,20 @@ def test_item_shards_and_peer_tables_host_side():
     assert (f.world, f.rank, f.flags[2]) == (3, 2, 48)
     # scratch sizing of the shard evaluator is CUDA-free except for the SM count: monotone in the batch
     assert ctypes.sizeof(_C.PeerItems) == 8 + 5 * 8 * _C.MAX_PEERS
+
+
+def test_step_entry_points_take_an_empty_batch_without_index_pointers():
+    """A rank whose share of the global batch is empty passes empty index tensors, and torch gives an empty tensor a null data
+    pointer: the step entry points accept B = 0 without indices (and launch nothing); B > 0 still needs them."""
+    import ctypes
+    from hassaku_b200 import _C
+    lib = _C.lib()
+    t = _C.MfTables(0x1000, 0x2000, None, None, None, 4, 4, 4, 4)
+    g = _C.MfTables(0x3000, 0x4000, None, None, None, 4, 4, 4, 4)
+    p = _C.make_peer_items([0x2000, 0x5000], [0x4000, 0x6000])
+    for B, rc in ((0, 0), (3, -1)):
+        assert lib.hsk_mf_train_fused_v(ctypes.byref(t), ctypes.byref(g), None, None, B, 6, 8, 0, 0.0, None, None, None,
+                                        None, 0, None) == rc
+        assert lib.hsk_mf_train_fused_peer(ctypes.byref(t), ctypes.byref(g), ctypes.byref(p), None, None, B, 6, 8, 0, 0.0, None,
+                                           1, None, None, None) == rc
+    assert b'null' in lib.hsk_last_error()
