@@ -103,6 +103,7 @@ def _declare(lib):
         'hsk_route_items': (i32, [vp, i64, i64, i32, i32, i32, vp, vp, vp, vp, i64, vp, vp]),
         'hsk_shard_pack': (i32, [vp, vp, i32, i64, vp, i32, i32, vp, vp, vp]),
         'hsk_shard_unpack_add': (i32, [vp, i32, i64, vp, i32, i32, vp, vp, vp, i64, vp, vp, vp]),
+        'hsk_shard_unpack_ordered': (i32, [vp, i32, i64, vp, i32, i32, vp, vp, vp, i64, vp, vp, vp]),
         'hsk_adamw_dense': (i32, [vp, vp, vp, vp, i64, f64, f64, f64, f64, f64, i64, i32, i32, i32, vp]),
         'hsk_sample_negatives': (i32, [vp, vp, i32, i32, i64, i64, vp, vp, C.c_uint64, C.c_uint64, i32, vp, vp, vp, vp]),
         'hsk_adagrad_dense': (i32, [vp, vp, vp, i64, f64, f64, f64, i32, vp]),
@@ -127,6 +128,7 @@ def _declare(lib):
         'hsk_det_scratch_bytes': (i64, [i32, i32, i32]),
         'hsk_mf_scatter_grads_det': (i32, [T, T, vp, vp, vp, i32, i32, vp, i64, vp, vp]),
         'hsk_mf_train_fused_det': (i32, [T, T, vp, vp, i32, i32, i32, f32, vp, vp, vp, vp, i64, vp, vp]),
+        'hsk_mf_train_fused_det_n': (i32, [T, T, vp, vp, i32, i32, i64, i32, f32, vp, vp, vp, vp, i64, vp, vp]),
         'hsk_rec_loss_det': (i32, [vp, vp, i32, i32, i32, f32, f32, vp, vp, vp, vp, i64, vp]),
         'hsk_rank_metrics_sums_det': (i32, [vp, i32, i32, vp, vp, i32, vp, vp]),
         'hsk_mf_train_fused_pack': (i32, [T, T, i64, i32, vp, i32, vp, vp, i32, i32, i32, f32, vp, vp, vp]),
@@ -398,17 +400,21 @@ def shard_pack(V2d, Ib, rows, world: int, capq: int, out, status=None):
                                     _ptr(status), st), 'hsk_shard_pack')
 
 
-def shard_unpack_add(inp, rows, world: int, capq: int, gV2d, gIb=None, stamps=None, step: int = 0, step_dev=None, status=None):
+def shard_unpack_add(inp, rows, world: int, capq: int, gV2d, gIb=None, stamps=None, step: int = 0, step_dev=None, status=None,
+                     ordered: bool = False):
+    """Owner side of the sparse exchange: the peers' row / bias gradients into gV2d / gIb, rows stamped.  `ordered`:
+    hsk_shard_unpack_ordered (every row composed in increasing rank order and stored, no atomics) instead of
+    hsk_shard_unpack_add."""
     _req(rows, torch.int32, 'rows'); _req(inp, torch.float32, 'inp')
     ld = gV2d.stride(0)
     if stamps is not None:
         _req(stamps, torch.uint8, 'stamps')
     if step_dev is not None:
         _req(step_dev, torch.int64, 'step_dev')
+    name = 'hsk_shard_unpack_ordered' if ordered else 'hsk_shard_unpack_add'
     with _on_device_of(inp, rows, gV2d, gIb, stamps, step_dev, status) as st:
-        _check(lib().hsk_shard_unpack_add(inp.data_ptr(), ld, gV2d.shape[0], rows.data_ptr(), world, capq, gV2d.data_ptr(),
-                                          _ptr(gIb), _ptr(stamps), step, _ptr(step_dev), _ptr(status), st),
-               'hsk_shard_unpack_add')
+        _check(getattr(lib(), name)(inp.data_ptr(), ld, gV2d.shape[0], rows.data_ptr(), world, capq, gV2d.data_ptr(),
+                                    _ptr(gIb), _ptr(stamps), step, _ptr(step_dev), _ptr(status), st), name)
 
 
 def adamw_dense(p, m, v, g, lr, beta1, beta2, eps, weight_decay, step: int, arith: int = 0, adam_l2: bool = False,
@@ -863,15 +869,22 @@ def mf_scatter_grads_det(tables: MfTables, grads: MfTables, u_idx, i_idx, dscore
 
 
 def mf_train_fused_det(tables: MfTables, grads: MfTables, u_idx, i_idx, loss_kind: int, neg_shift: float, loss_accum,
-                       scratch, scores_out=None, dscores_out=None, status=None):
-    """hsk_mf_train_fused_det: the fused step with per-sample dL/ds and a fixed-order scatter / loss sum."""
+                       scratch, scores_out=None, dscores_out=None, status=None, B_global: Optional[int] = None):
+    """hsk_mf_train_fused_det: the fused step with per-sample dL/ds and a fixed-order scatter / loss sum.  `B_global`: the
+    normalisers of a global batch this one is a share of (hsk_mf_train_fused_det_n, the sharded 'ordered' step)."""
     _req(u_idx, torch.int64, 'u_idx'); _req(i_idx, torch.int64, 'i_idx'); _req(loss_accum, torch.float64, 'loss_accum')
     B, N1 = i_idx.shape
     with _on_device_of(u_idx, i_idx, loss_accum, scratch, scores_out, dscores_out, status) as st:
-        _check(lib().hsk_mf_train_fused_det(C.byref(tables), C.byref(grads), u_idx.data_ptr(), i_idx.data_ptr(), B, N1,
-                                            loss_kind, neg_shift, loss_accum.data_ptr(), _ptr(scores_out),
-                                            _ptr(dscores_out), scratch.data_ptr(), _scratch_bytes(scratch), _ptr(status),
-                                            st), 'hsk_mf_train_fused_det')
+        if B_global is None:
+            _check(lib().hsk_mf_train_fused_det(C.byref(tables), C.byref(grads), u_idx.data_ptr(), i_idx.data_ptr(), B, N1,
+                                                loss_kind, neg_shift, loss_accum.data_ptr(), _ptr(scores_out),
+                                                _ptr(dscores_out), scratch.data_ptr(), _scratch_bytes(scratch), _ptr(status),
+                                                st), 'hsk_mf_train_fused_det')
+        else:
+            _check(lib().hsk_mf_train_fused_det_n(C.byref(tables), C.byref(grads), u_idx.data_ptr(), i_idx.data_ptr(), B, N1,
+                                                  B_global, loss_kind, neg_shift, loss_accum.data_ptr(), _ptr(scores_out),
+                                                  _ptr(dscores_out), scratch.data_ptr(), _scratch_bytes(scratch), _ptr(status),
+                                                  st), 'hsk_mf_train_fused_det_n')
 
 
 def rec_loss_det(scores, labels, loss_kind: int, neg_shift: float, grad_scale: float, loss_accum, dscores, scratch,

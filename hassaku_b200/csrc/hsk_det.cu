@@ -7,6 +7,7 @@
 //                              (samples), one fixed-order segmented reduction per distinct row, plain stores
 //   hsk_mf_train_fused_det     forward + loss + dL/ds per sample (same arithmetic as the fused kernels, dL/ds to scratch,
 //                              per-sample fp64 loss), then the scatter above and a fixed-order loss sum
+//   hsk_mf_train_fused_det_n   the same with a global normaliser: one rank's share of the sharded 'ordered' step
 //   hsk_rec_loss_det           hsk_rec_loss with the per-row losses summed in a fixed order
 //   hsk_rank_metrics_sums_det  fixed-order sum of per-user metric rows into the per-group sums
 //   hsk_rank_metrics_sums_det_pack  the same for every active trial of a trial pack, batch by batch
@@ -645,17 +646,20 @@ extern "C" int hsk_mf_scatter_grads_det(const hsk_mf_tables* t, const hsk_mf_tab
     return det_scatter(a, dscores, static_cast<char*>(scratch), p, as_stream(stream));
 }
 
-extern "C" int hsk_mf_train_fused_det(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx,
-                                      int B, int N1, int loss_kind, float neg_shift, double* loss_accum, float* scores_out,
-                                      float* dscores_out, void* scratch, int64_t scratch_bytes, int32_t* status,
-                                      hsk_stream_t stream) {
+// B_global: the loss / gradient normaliser (the whole step's batch when this is one rank's share of it); the forward,
+// sorts, scatter and loss sum run on the local B
+static int train_fused_det(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx, int B,
+                           int N1, int64_t B_global, int loss_kind, float neg_shift, double* loss_accum, float* scores_out,
+                           float* dscores_out, void* scratch, int64_t scratch_bytes, int32_t* status, hsk_stream_t stream,
+                           const char* who) {
     TrainArgs a;
     DetPlan p;
-    int rc = det_args(a, t, g, u_idx, i_idx, B, N1, scratch, scratch_bytes, p, "hsk_mf_train_fused_det");
+    int rc = det_args(a, t, g, u_idx, i_idx, B, N1, scratch, scratch_bytes, p, who);
     if (rc) return rc;
-    HSK_REQUIRE(loss_kind >= 0 && loss_kind <= 2, "hsk_mf_train_fused_det: unknown loss kind %d", loss_kind);
-    HSK_REQUIRE(loss_kind != HSK_LOSS_BPR || N1 >= 2, "hsk_mf_train_fused_det: bpr needs at least one negative");
-    HSK_REQUIRE(N1 <= 10240, "hsk_mf_train_fused_det: at most 10240 slots per sample");
+    HSK_REQUIRE(loss_kind >= 0 && loss_kind <= 2, "%s: unknown loss kind %d", who, loss_kind);
+    HSK_REQUIRE(loss_kind != HSK_LOSS_BPR || N1 >= 2, "%s: bpr needs at least one negative", who);
+    HSK_REQUIRE(N1 <= 10240, "%s: at most 10240 slots per sample", who);
+    HSK_REQUIRE(B_global >= B && B_global <= 0x7FFFFFFFll, "%s: need B <= B_global < 2^31", who);
     if (B == 0) return HSK_OK;
     a.status = status; a.loss_kind = loss_kind; a.neg_shift = neg_shift;
     a.scores_out = scores_out; a.dscores_out = dscores_out;
@@ -665,11 +669,35 @@ extern "C" int hsk_mf_train_fused_det(const hsk_mf_tables* t, const hsk_mf_table
     cudaStream_t s = as_stream(stream);
     const int nv = (a.nvec + 31) / 32;
     const size_t smem = sizeof(float) * (size_t)N1;
-    HSK_DISPATCH_NV(nv, (det_forward_kernel<NV><<<B, kWarpsPerCta * 32, smem, s>>>(a, ds, loss_rows)));
-    rc = check_launch("hsk_mf_train_fused_det");
+    // det_forward_kernel reads a.B only as loss_row's normaliser (the sample is blockIdx.x): the grid stays the local B
+    TrainArgs fa = a;
+    fa.B = (int)B_global;
+    HSK_DISPATCH_NV(nv, (det_forward_kernel<NV><<<B, kWarpsPerCta * 32, smem, s>>>(fa, ds, loss_rows)));
+    rc = check_launch(who);
     if (rc) return rc;
     if (loss_accum) det_loss_sum_kernel<<<1, 256, 0, s>>>(loss_rows, B, loss_accum);
     return det_scatter(a, ds, base, p, s);
+}
+
+extern "C" int hsk_mf_train_fused_det(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx,
+                                      int B, int N1, int loss_kind, float neg_shift, double* loss_accum, float* scores_out,
+                                      float* dscores_out, void* scratch, int64_t scratch_bytes, int32_t* status,
+                                      hsk_stream_t stream) {
+    return train_fused_det(t, g, u_idx, i_idx, B, N1, B, loss_kind, neg_shift, loss_accum, scores_out, dscores_out, scratch,
+                           scratch_bytes, status, stream, "hsk_mf_train_fused_det");
+}
+
+extern "C" int hsk_mf_train_fused_det_n(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx,
+                                        int B, int N1, int64_t B_global, int loss_kind, float neg_shift, double* loss_accum,
+                                        float* scores_out, float* dscores_out, void* scratch, int64_t scratch_bytes,
+                                        int32_t* status, hsk_stream_t stream) {
+    static const int64_t kNoIndex = 0;
+    if (B == 0) {     // a rank without samples in this step: nothing is launched, its (empty) index arrays may be null
+        if (!u_idx) u_idx = &kNoIndex;
+        if (!i_idx) i_idx = &kNoIndex;
+    }
+    return train_fused_det(t, g, u_idx, i_idx, B, N1, B_global, loss_kind, neg_shift, loss_accum, scores_out, dscores_out,
+                           scratch, scratch_bytes, status, stream, "hsk_mf_train_fused_det_n");
 }
 
 extern "C" int hsk_rec_loss_det(const float* scores, const double* labels, int B, int N1, int loss_kind, float neg_shift,

@@ -11,6 +11,8 @@
 //   hsk_shard_pack      owner: the rows (and item biases) the peers asked for -> send blocks [G, block_rows, ld]
 //   hsk_shard_unpack_add owner: row / bias gradients received back -> added into the dense gradient table, rows stamped
 //                       for hsk_adamw_dense_rows
+//   hsk_shard_unpack_ordered  the same with the contributions of one row composed in increasing rank order and stored (no
+//                       atomics): the owner side of the deterministic 'ordered' exchange
 //
 // One exchange block per peer is [block_rows, ld] floats: rows [0, capq) are item rows, the floats from row capq on hold
 // the capq item biases flat, block_rows = capq + ceil(capq / ld) — so ONE all-to-all moves rows and biases.
@@ -192,6 +194,82 @@ __global__ void __launch_bounds__(256) shard_unpack_add_kernel(const float* __re
     }
 }
 
+// rank-ordered variant (contract in include/hassaku_b200.h, hsk_shard_unpack_ordered): slot of local row r in peer q2's
+// request list rows[q2, 0 .. capq) — ascending local rows, then -1 padding — or -1
+__device__ __forceinline__ int find_row(const int32_t* __restrict__ list, int capq, int32_t r) {
+    int lo = 0, hi = capq;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        const int32_t v = __ldg(list + mid);
+        if (v >= 0 && v < r) lo = mid + 1; else hi = mid;
+    }
+    return lo < capq && __ldg(list + lo) == r ? lo : -1;
+}
+
+__device__ __forceinline__ float4 fadd4_rn(float4 a, float4 b) {
+    return make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
+}
+
+// one warp per request entry (q, k); only the entry of the LOWEST rank that fetched the row does the work: it stores that
+// rank's contribution, then adds the later ranks' contributions in rank order (their slots found by binary search, 32 ranks
+// per round, one per lane) and stamps the row.  Every row has one writer and a fixed summation order: no atomics.
+__global__ void __launch_bounds__(256) shard_unpack_ordered_kernel(const float* __restrict__ in, int ld, int64_t n_local,
+                                                                   const int32_t* __restrict__ rows, int G, int capq,
+                                                                   int64_t block_rows, float* __restrict__ gV,
+                                                                   float* __restrict__ gIb, uint8_t* __restrict__ stamps,
+                                                                   int stamp_host, const int64_t* __restrict__ step_dev,
+                                                                   int32_t* status) {
+    __shared__ int s_slot[8][32];
+    const int nvec = ld >> 2;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t total = (int64_t)G * capq;
+    const uint8_t stamp = (uint8_t)(step_dev ? 1 + (int)(*step_dev % 255) : stamp_host);
+    for (int64_t e = (int64_t)blockIdx.x * 8 + warp; e < total; e += (int64_t)gridDim.x * 8) {
+        const int32_t r = rows[e];
+        if (r < 0) continue;
+        if (r >= n_local) {
+            if (lane == 0 && status) atomicOr(status, HSK_STATUS_BAD_INDEX);
+            continue;
+        }
+        const int q = (int)(e / capq), k = (int)(e - (int64_t)q * capq);
+        bool lower = false;              // a lower rank fetched the row too: its entry is the writer
+        for (int b = 0; b < q && !lower; b += 32)
+            lower = __any_sync(kFull, b + lane < q && find_row(rows + (int64_t)(b + lane) * capq, capq, r) >= 0);
+        if (lower) continue;
+        const float4* own = reinterpret_cast<const float4*>(in + ((int64_t)q * block_rows + k) * ld);
+        float4* dp = reinterpret_cast<float4*>(gV + (int64_t)r * ld);
+        float bias = gIb ? in[((int64_t)q * block_rows + capq) * ld + k] : 0.f;
+        int b = q + 1;
+        do {                             // ranks b .. b + 31 (the first round also stores this rank's contribution)
+            const int q2 = b + lane;
+            const int slot = q2 < G ? find_row(rows + (int64_t)q2 * capq, capq, r) : -1;
+            unsigned found = __ballot_sync(kFull, slot >= 0);
+            s_slot[warp][lane] = slot;
+            __syncwarp();
+            for (int t = lane; t < nvec; t += 32) {
+                float4 acc = b == q + 1 ? own[t] : dp[t];
+                for (unsigned m = found; m; m &= m - 1) {
+                    const int j = __ffs(m) - 1;
+                    const float4* sp = reinterpret_cast<const float4*>(in + ((int64_t)(b + j) * block_rows + s_slot[warp][j]) * ld);
+                    acc = fadd4_rn(acc, sp[t]);
+                }
+                dp[t] = acc;
+            }
+            if (gIb && lane == 0)
+                for (unsigned m = found; m; m &= m - 1) {
+                    const int j = __ffs(m) - 1;
+                    bias = __fadd_rn(bias, in[((int64_t)(b + j) * block_rows + capq) * ld + s_slot[warp][j]]);
+                }
+            __syncwarp();
+            b += 32;
+        } while (b < G);
+        if (lane == 0) {
+            if (gIb) gIb[r] = bias;
+            if (stamps) stamps[r] = stamp;
+        }
+    }
+}
+
 static inline int64_t cap_padded(int64_t n_items, int G) {
     const int64_t cap = (n_items + G - 1) / G;
     return (cap + kScanBlock - 1) / kScanBlock * kScanBlock;
@@ -267,4 +345,17 @@ extern "C" int hsk_shard_unpack_add(const float* in, int ld, int64_t n_local, co
     shard_unpack_add_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, as_stream(stream)>>>(
         in, ld, n_local, rows, G, capq, hsk_shard_block_rows(capq, ld), gV, gIb, stamps, hsk_row_stamp(step), step_dev, status);
     return check_launch("hsk_shard_unpack_add");
+}
+
+extern "C" int hsk_shard_unpack_ordered(const float* in, int ld, int64_t n_local, const int32_t* rows, int G, int capq, float* gV,
+                                        float* gIb, uint8_t* stamps, int64_t step, const int64_t* step_dev, int32_t* status,
+                                        hsk_stream_t stream) {
+    HSK_REQUIRE(in && rows && gV, "hsk_shard_unpack_ordered: null pointer");
+    HSK_REQUIRE(ld >= 4 && ld % 4 == 0 && aligned16(in) && aligned16(gV) && G >= 1 && capq >= 1 && n_local >= 0,
+                "hsk_shard_unpack_ordered: bad sizes / alignment");
+    const int64_t total = (int64_t)G * capq;
+    int64_t blocks = (total + 7) / 8, cap = (int64_t)sm_count() * 16;
+    shard_unpack_ordered_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, as_stream(stream)>>>(
+        in, ld, n_local, rows, G, capq, hsk_shard_block_rows(capq, ld), gV, gIb, stamps, hsk_row_stamp(step), step_dev, status);
+    return check_launch("hsk_shard_unpack_ordered");
 }

@@ -18,6 +18,10 @@ graph (`exchange='sparse_graph'`):
   5. all-to-all: compact row / bias gradients to the owners, hsk_shard_unpack_add into the local dense gradient
   6. hsk_adamw_dense_rows over the local arena: 24 B / parameter for rows without a gradient, 32 B for the touched ones
      (the dominant term of the step shards perfectly: P / G parameters per GPU)
+ORDERED exchange (`exchange='ordered'` / `'ordered_graph'`): the sparse exchange with every floating-point cross-row and
+cross-rank reduction in a fixed order — hsk_mf_train_fused_det_n in step 4, hsk_shard_unpack_ordered in step 5, the
+global-bias gradient and the loss summed in rank order — so a run gives the same bits every time at a fixed world size
+(order contract in include/hassaku_b200.h); the exchange to use under torch.use_deterministic_algorithms(True).
 DENSE exchange (cfg2: the batch covers the item table anyway): one all-gather of the [cap + bias rows, ld] blocks into a
 rank-major replica, the ordinary fused kernel, one reduce-scatter of the dense gradient block.
 PEER exchange (one NVLink / NVSwitch node, rows <= 128 floats; `exchange='peer'` / `'peer_graph'`): no exchange buffers at all.
@@ -82,6 +86,9 @@ class CudaOps:
     def unpack_add(self, inp, rows, world, capq, gV2d, gIb, stamps, step, step_dev):
         _C.shard_unpack_add(inp, rows, world, capq, gV2d, gIb, stamps, step, step_dev, self.status)
 
+    def unpack_ordered(self, inp, rows, world, capq, gV2d, gIb, stamps, step, step_dev):
+        _C.shard_unpack_add(inp, rows, world, capq, gV2d, gIb, stamps, step, step_dev, self.status, ordered=True)
+
     def mark_rows(self, idx, n_rows, stamps, step, step_dev):
         _C.mark_rows(idx, n_rows, stamps, step, step_dev)
 
@@ -92,6 +99,19 @@ class CudaOps:
         t = _C.make_tables(Uw, Vc[:, :lay.d], Ub, Ibc, Gb, lay.d)
         g = _C.make_tables(gU, gVc[:, :lay.d], gUb, gIbc, gGb, lay.d)
         _C.mf_train_fused_n(t, g, u_local, compact_idx, B_global, kind, shift, loss_accum, self.status)
+
+    def det_scratch_bytes(self, B, N1, ld):
+        return _C.det_scratch_bytes(B, N1, ld)
+
+    def train_fused_det(self, lay: ArenaLayout, arena, g_arena, Vc, Ibc, gVc, gIbc, u_local, compact_idx, B_global, kind, shift,
+                        loss_accum, scratch, dscores_out=None):
+        """train_fused in the fixed order of deterministic mode (hsk_mf_train_fused_det_n): touched rows are STORED."""
+        Uw, _, Ub, _, Gb = lay.views(arena)
+        gU, _, gUb, _, gGb = lay.views(g_arena)
+        t = _C.make_tables(Uw, Vc[:, :lay.d], Ub, Ibc, Gb, lay.d)
+        g = _C.make_tables(gU, gVc[:, :lay.d], gUb, gIbc, gGb, lay.d)
+        _C.mf_train_fused_det(t, g, u_local, compact_idx, kind, shift, loss_accum, scratch, dscores_out=dscores_out,
+                              status=self.status, B_global=B_global)
 
     def train_fused_peer(self, lay: ArenaLayout, arena, g_arena, peers, n_items_global, u_local, i_global, B_global, kind, shift,
                          loss_accum, step, step_dev):
@@ -135,6 +155,8 @@ class ShardedMF:
         self.stamp_users = torch.zeros(max(self.spec.n_local_users, 1), dtype=torch.uint8, device=self.device)
         self.stamp_items = torch.zeros(max(self.spec.n_local_items, 1), dtype=torch.uint8, device=self.device)
         self._sparse, self._dense, self._graphs = {}, None, {}
+        self._ordered = {}
+        self._rank_ordered_loss = False     # set by the ordered exchange: pop_loss sums the ranks' losses in rank order
         self._peer = None
         self._ipc = {}          # (rank, IPC handle) -> base address here of a peer's allocation (opened once, closed in close())
 
@@ -154,6 +176,31 @@ class ShardedMF:
     def _all_reduce(self, t: torch.Tensor, op=None):
         if self.spec.world > 1:
             dist.all_reduce(t, op=op if op is not None else dist.ReduceOp.SUM, group=self.group)
+
+    def _rank_ordered_sum(self, t: torch.Tensor):
+        """t = the ranks' values of t added in rank order, starting from rank 0's (all-gather, then G - 1 adds): the same
+        bits on every run, where an all-reduce's summation order depends on the collective's algorithm."""
+        G = self.spec.world
+        if G == 1:
+            return
+        every = torch.empty((G,) + tuple(t.shape), dtype=t.dtype, device=t.device)
+        self._all_gather(every, t.contiguous())
+        t.copy_(every[0])
+        for q in range(1, G):
+            t.add_(every[q])
+
+    def _reduce_metric_sums(self, evaluator):
+        """The evaluator's per-rank metric sums and counts summed over the ranks; under torch.use_deterministic_algorithms
+        the floating-point sums are added in rank order (every rank's evaluator already sums in a fixed order there)."""
+        det = determinism.enabled()
+        for name in ('_sums', '_counts', '_hit_sums'):
+            x = getattr(evaluator, name, None)
+            if x is None:
+                continue
+            if det and x.is_floating_point():
+                self._rank_ordered_sum(x)
+            else:
+                self._all_reduce(x)
 
     def _reduce_scatter(self, out: torch.Tensor, inp: torch.Tensor):
         if self.spec.world == 1:
@@ -222,18 +269,28 @@ class ShardedMF:
 
     # ---- SPARSE exchange: fixed-capacity padded all-to-alls, device-side routing ----
     def _sparse_buffers(self, n_slots: int, capq: Optional[int]):
+        return self._exchange_buffers(self._sparse, n_slots, capq)
+
+    def _exchange_buffers(self, store: dict, n_slots: int, capq: Optional[int], shape=None):
+        """The sparse exchange's buffers for one batch shape (`store`: the buffer sets of one exchange).  `shape` (B, N1):
+        the ordered exchange's set, which also holds the compact index and the deterministic step's scratch — a captured
+        graph holds their addresses, so a graph of an evicted set is dropped with it."""
         G, lay, dev = self.spec.world, self.layout, self.device
         capq = capq or exchange_capacity(n_slots, self.spec.n_items, G)
-        key = (n_slots, capq)
-        if key not in self._sparse:
-            if len(self._sparse) >= 2:      # a new batch shape (e.g. the epoch's tail batch): keep at most two sets of buffers
-                self._sparse.pop(next(iter(self._sparse)))
+        key = (n_slots, capq) if shape is None else (tuple(shape), capq)
+        if key not in store:
+            if len(store) >= 2:      # a new batch shape (e.g. the epoch's tail batch): keep at most two sets of buffers
+                old = next(iter(store))
+                store.pop(old)
+                if shape is not None:
+                    for gk in [k for k in self._graphs if k[0] == 'ordered' and k[1] == old[0]]:
+                        self._drop_graph(gk)
             ld = lay.ld
             br = capq + math.ceil(capq / ld)                       # == hsk_shard_block_rows(capq, ld)
             z = lambda shape, dt=torch.float32: torch.zeros(shape, dtype=dt, device=dev)
             n_scr = _C.route_scratch_bytes(self.spec.n_items, G) if dev.type == 'cuda' else 16
             grads = z(G * br * ld + G * br)                         # [gVc | gIbc]: one memset per step
-            self._sparse[key] = {
+            store[key] = {
                 'capq': capq, 'br': br,
                 'req_rows': z((G, capq), torch.int32), 'req_count': z(G, torch.int32),
                 'recv_rows': z((G, capq), torch.int32), 'scratch': z(n_scr, torch.uint8),
@@ -241,7 +298,11 @@ class ShardedMF:
                 'grads': grads, 'gVc': grads[:G * br * ld].view(G * br, ld), 'gIbc': grads[G * br * ld:],
                 'recv_g': z((G, br, ld)),
             }
-        return self._sparse[key]
+            if shape is not None:
+                B, N1 = shape
+                store[key]['compact_idx'] = z((B, N1), torch.int64)
+                store[key]['det'] = z(max(self.ops.det_scratch_bytes(B, N1, ld), 16), torch.uint8)
+        return store[key]
 
     def _sparse_body(self, u_global, i_global, B_global, loss_kind, neg_shift, lr, wd, decoupled, capq=None, consts_dev=None,
                      step_dev=None):
@@ -287,6 +348,55 @@ class ShardedMF:
         """u_global int64 [B_r] (all owned by this rank: u % G == rank), i_global int64 [B_r, 1+N] global item ids."""
         self._sparse_body(u_global, i_global.contiguous(), B_global, loss_kind, neg_shift, lr, wd, decoupled, capq)
         self.t += 1
+
+    # ---- ORDERED exchange: the sparse exchange with every cross-row and cross-rank float reduction in a fixed order
+    # (order contract of the sharded step, include/hassaku_b200.h): bitwise reproducible at a fixed world size ----
+    def _ordered_body(self, u_global, i_global, B_global, loss_kind, neg_shift, lr, wd, decoupled, capq=None, consts_dev=None,
+                      step_dev=None):
+        """_sparse_body with hsk_mf_train_fused_det_n instead of the atomic fused kernel, hsk_shard_unpack_ordered instead
+        of the atomic unpack-add, and the global-bias gradient summed in rank order instead of by an all-reduce."""
+        G, lay = self.spec.world, self.layout
+        ld = lay.ld
+        S = self._exchange_buffers(self._ordered, i_global.numel(), capq, shape=i_global.shape)
+        capq, br = S['capq'], S['br']
+        _, _, _, Ib, _ = lay.views(self.arena)
+        has_ib = Ib is not None
+        step = self.t + 1
+        self._rank_ordered_loss = True
+        compact_idx = S['compact_idx']
+        self.ops.route(i_global, self.spec.n_items, G, capq, ld, S['req_rows'], S['req_count'], compact_idx, S['scratch'])
+        self._a2a(S['recv_rows'], S['req_rows'])
+        self.ops.pack(self._table2d(self.arena, 'V'), Ib.view(-1) if has_ib else None, S['recv_rows'], G, capq, S['send'])
+        self._a2a(S['Vc'].view(G, br, ld), S['send'])
+        if has_ib:
+            S['Ibc'].view(G, br)[:, :capq] = S['Vc'].view(G, br * ld)[:, capq * ld:capq * ld + capq]
+        S['grads'].zero_()
+        u_local = self.ops.local_index(u_global, G, 0)
+        self.ops.mark_rows(u_local, lay.n_users, self.stamp_users, step, step_dev)
+        self.ops.train_fused_det(lay, self.arena, self.g, S['Vc'], S['Ibc'] if has_ib else None, S['gVc'],
+                                 S['gIbc'] if has_ib else None, u_local, compact_idx, B_global, _C.LOSS_KINDS[loss_kind],
+                                 neg_shift, self.loss_accum, S['det'])
+        if has_ib:
+            S['gVc'].view(G, br * ld)[:, capq * ld:capq * ld + capq] = S['gIbc'].view(G, br)[:, :capq]
+        self._a2a(S['recv_g'], S['gVc'].view(G, br, ld))
+        gIb = lay.views(self.g)[3]
+        self.ops.unpack_ordered(S['recv_g'], S['recv_rows'], G, capq, self._table2d(self.g, 'V'),
+                                gIb.view(-1) if gIb is not None else None, self.stamp_items, step, step_dev)
+        gGb = lay.views(self.g)[4]
+        if gGb is not None:
+            self._rank_ordered_sum(gGb)
+        self.ops.adamw(self.arena, self.m, self.v, self.g, self._segments(True, True), lr, wd, step, decoupled,
+                       consts_dev=consts_dev, step_dev=step_dev)
+
+    def train_step_ordered(self, u_global: torch.Tensor, i_global: torch.Tensor, B_global: int, loss_kind: str,
+                           neg_shift: float, lr: float, wd: float, decoupled: bool = True, capq: Optional[int] = None):
+        """The step with the ORDERED exchange (see _ordered_body): the same bits on every run at a fixed world size, with or
+        without torch.use_deterministic_algorithms."""
+        self._ordered_body(u_global, i_global.contiguous(), B_global, loss_kind, neg_shift, lr, wd, decoupled, capq)
+        self.t += 1
+
+    def train_step_ordered_graphed(self, *a, capq=None):
+        return self._graphed(self._ordered_body, 'ordered', *a, capq)
 
     # ---- DENSE exchange: when the batch touches (nearly) every item anyway ----
     def _dense_buffers(self):
@@ -546,22 +656,30 @@ class ShardedMF:
 
     def step(self, u_global, i_global, B_global, loss_kind, neg_shift, lr, wd, decoupled=True, exchange='auto', capq=None):
         """Dispatch on the expected fraction of distinct items: dense exchange when the batch covers the item table.
-        Raises under torch.use_deterministic_algorithms(True) (warns under warn_only): the exchanges reduce gradients
-        from several ranks with floating-point atomics, and there is no deterministic implementation yet."""
-        determinism.alert_not_deterministic('ShardedMF.step')
+        `exchange='ordered'` / `'ordered_graph'` is the deterministic step (bitwise reproducible at a fixed world size);
+        every other exchange reduces gradients from several ranks with floating-point atomics, so it raises under
+        torch.use_deterministic_algorithms(True) (warns under warn_only)."""
+        if exchange not in ('ordered', 'ordered_graph'):
+            determinism.alert_not_deterministic(f"ShardedMF.step(exchange={exchange!r}; exchange='ordered' is the "
+                                                "deterministic one)")
         if exchange in ('auto', 'auto_graph'):
             dense = i_global.numel() >= 2 * self.spec.n_items // self.spec.world
             exchange = ('dense' if dense else 'sparse') + ('_graph' if exchange == 'auto_graph' else '')
         fn = {'dense': self.train_step_dense, 'dense_graph': self.train_step_dense_graphed, 'sparse': self.train_step,
               'sparse_graph': self.train_step_graphed, 'peer': self.train_step_peer,
-              'peer_graph': self.train_step_peer_graphed}[exchange]
+              'peer_graph': self.train_step_peer_graphed, 'ordered': self.train_step_ordered,
+              'ordered_graph': self.train_step_ordered_graphed}[exchange]
         with nvtx.range('hsk.sharded_step'):
             return fn(u_global, i_global, B_global, loss_kind, neg_shift, lr, wd, decoupled, capq=capq)
 
     def pop_loss(self) -> float:
-        """Sum over ranks of the batch-mean loss contributions since the last call (one all-reduce + host sync)."""
+        """Sum over ranks of the batch-mean loss contributions since the last call (one all-reduce + host sync; after an
+        ordered step or under torch.use_deterministic_algorithms an all-gather summed in rank order)."""
         t = self.loss_accum.clone()
-        self._all_reduce(t)
+        if self._rank_ordered_loss or determinism.enabled():
+            self._rank_ordered_sum(t)
+        else:
+            self._all_reduce(t)
         self.loss_accum.zero_()
         return float(t.item())
 
@@ -729,11 +847,8 @@ class ShardedMF:
                 merge(j)                 # comm stream: runs under score(j + 1)
         if use_streams:
             main.wait_stream(comm)
-        # one all-reduce of the accumulators per sweep
-        self._all_reduce(evaluator._sums)
-        self._all_reduce(evaluator._counts)
-        if getattr(evaluator, '_hit_sums', None) is not None:
-            self._all_reduce(evaluator._hit_sums)
+        # one reduction of the accumulators per sweep
+        self._reduce_metric_sums(evaluator)
         return evaluator.get_results()
 
 
@@ -802,10 +917,7 @@ class ShardedMF:
                 if kc > k:
                     _C.rescore_topk(t, rows_l, ci, k, top_s[:n], top_i[:n], status=self.status, cand_scores=cs)
             evaluator.eval_batch_topk(gids, top_i[:n].contiguous(), labels)
-        self._all_reduce(evaluator._sums)
-        self._all_reduce(evaluator._counts)
-        if getattr(evaluator, '_hit_sums', None) is not None:
-            self._all_reduce(evaluator._hit_sums)
+        self._reduce_metric_sums(evaluator)
         return evaluator.get_results()
 
 
@@ -906,10 +1018,7 @@ class ShardedMF:
             if kc > k:
                 _C.rescore_topk_shards(t_user, shards, rows_l, ci, k, top_s[:n], top_i[:n], status=self.status, cand_scores=cs)
             evaluator.eval_batch_topk(gids, top_i[:n].contiguous(), labels)
-        self._all_reduce(evaluator._sums)
-        self._all_reduce(evaluator._counts)
-        if getattr(evaluator, '_hit_sums', None) is not None:
-            self._all_reduce(evaluator._hit_sums)
+        self._reduce_metric_sums(evaluator)
         torch.cuda.synchronize(dev)
         if G > 1:
             dist.barrier(group=self.group)                        # nobody still reads this rank's packed shard when it is freed

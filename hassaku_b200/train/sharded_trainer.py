@@ -12,7 +12,8 @@ Launch with torchrun (one rank per GPU); EVERY rank builds the same model / data
   * the item rows a rank needs are read from / their gradients reduced into the owners' memory by the step kernel over
     NVLink (`exchange='peer'`, one node, rows <= 128 floats) or exchanged by NCCL all-to-all (`'sparse'`) / all-gather +
     reduce-scatter (`'dense'`, batches that cover the item table) — chosen per shape unless `conf['sharded_exchange']` says
-    otherwise;
+    otherwise; `'ordered'` is the sparse exchange with every float reduction in a fixed order: with it, fit() under
+    torch.use_deterministic_algorithms(True) gives the same checkpoint, metrics and losses on every run at a fixed world size;
   * validation is the sharded full-rank evaluator (`ShardedMF.evaluate_replicated` while the item table fits one GPU, the
     item-sharded protocol otherwise): every rank gets the same metric dict, so early stopping needs no extra collective;
   * the best model is written by rank 0 as the reference's `model.pth` (full state_dict, reference key names / shapes).
@@ -41,7 +42,7 @@ MODEL_FILE = 'model.pth'
 
 
 class ShardedTrainer:
-    EXCHANGES = ('auto', 'peer', 'sparse', 'dense')
+    EXCHANGES = ('auto', 'peer', 'sparse', 'dense', 'ordered')
 
     def __init__(self, model: SGDMatrixFactorization, train_loader, val_loader, rec_loss, conf: dict, group=None):
         if not dist.is_initialized():

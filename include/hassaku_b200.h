@@ -132,7 +132,26 @@ HSK_API int hsk_scatter_add_rows(float* dst, int ld, const int64_t* idx, int64_t
  *   hsk_shard_pack    (owner) rows [G, capq] (what the peers sent after the id all-to-all) -> out [G, block_rows, ld]:
  *       block q = the requested rows of V, then from row capq on their item biases flat (Ib nullable).
  *   hsk_shard_unpack_add (owner) in [G, block_rows, ld] = the peers' row / bias gradients in the same layout:
- *       gV[row] += ..., gIb[row] += ..., stamps[row] = hsk_row_stamp(step) (nullable; for hsk_adamw_dense_rows). */
+ *       gV[row] += ..., gIb[row] += ..., stamps[row] = hsk_row_stamp(step) (nullable; for hsk_adamw_dense_rows).
+ *   hsk_shard_unpack_ordered (owner) the same arguments; every row's gradient is composed in a fixed order and STORED
+ *       (no floating-point atomics): see the order contract of the sharded 'ordered' step below.  It relies on what
+ *       hsk_route_items guarantees of every request list rows[q, :]: the local rows are strictly ascending, followed by
+ *       -1 padding only.
+ *
+ * ORDER CONTRACT of the sharded 'ordered' step (restated by tests/sharded_det_oracle.py: sharded_scatter_grads).  World G, item
+ * i on rank i % G as local row i / G, user u on rank u % G; rank r processes the samples of the global batch whose user it
+ * owns, in global batch order.
+ *   1. Per rank: the single-GPU order contract (deterministic mode, below) on the local batch, with users keyed by local
+ *      row and items keyed by their row in the compact table of fetched rows — owner-major, ascending local row within an
+ *      owner, i.e. ordered exactly as (i % G) * cap + i / G.  Normalisers are global (B_global, hsk_mf_train_fused_det_n).
+ *      The rank's user-row and user-bias gradients are final and stored.
+ *   2. At the owner (hsk_shard_unpack_ordered): an item row's gradient, and its bias gradient, is the contributions of
+ *      the ranks that fetched the row in increasing rank order: the first is stored, each later one added with fadd_rn.
+ *      Rows no rank fetched are neither written nor stamped; stamps as hsk_shard_unpack_add.
+ *   3. Global bias: every rank's chunked sum over its local slots (the contract below) is all-gathered and the G values
+ *      are summed in rank order, starting from rank 0's value.
+ *   4. Loss: every rank adds its fixed-order sum to its loss accumulator; the G fp64 accumulators are summed in rank order.
+ *   At G = 1 this is the single-GPU deterministic step: the compact numbering is monotone in the item id. */
 HSK_API int64_t hsk_shard_block_rows(int capq, int ld);
 HSK_API int64_t hsk_route_scratch_bytes(int64_t n_items, int G);
 HSK_API int hsk_route_items(const int64_t* i_idx, int64_t n, int64_t n_items, int G, int capq, int ld, int32_t* req_rows,
@@ -143,6 +162,10 @@ HSK_API int hsk_shard_pack(const float* V, const float* Ib /* nullable */, int l
 HSK_API int hsk_shard_unpack_add(const float* in, int ld, int64_t n_local, const int32_t* rows, int G, int capq, float* gV,
                                  float* gIb /* nullable */, uint8_t* stamps /* nullable */, int64_t step,
                                  const int64_t* step_dev /* nullable: overrides step */, int32_t* status, hsk_stream_t stream);
+HSK_API int hsk_shard_unpack_ordered(const float* in, int ld, int64_t n_local, const int32_t* rows, int G, int capq, float* gV,
+                                     float* gIb /* nullable */, uint8_t* stamps /* nullable */, int64_t step,
+                                     const int64_t* step_dev /* nullable: overrides step */, int32_t* status,
+                                     hsk_stream_t stream);
 
 /* ---- evaluation over item SHARDS that stay where they are (one NVLink / NVSwitch node): every rank evaluates ITS users
  * against ALL items, streaming the other ranks' packed item tables straight from their HBM (TMA loads over peer mappings,
@@ -504,6 +527,9 @@ HSK_API int hsk_rank_metrics_sums_det_pack(const float* per_user, int Be, int ba
  *   hsk_mf_train_fused_det     = hsk_mf_train_fused: per sample the fused kernels' scores, loss term and dL/ds (a sample
  *       with an out-of-range index is skipped: dL/ds 0, loss 0), then the scatter above; *loss_accum += the per-sample
  *       fp64 losses summed in a fixed order.  N1 <= 10240.
+ *   hsk_mf_train_fused_det_n   = hsk_mf_train_fused_det with the loss / gradient normalisers of a global batch of
+ *       B_global >= B samples (as hsk_mf_train_fused_n): one rank's share of the sharded 'ordered' step.  B = 0 (a rank
+ *       without samples) launches nothing and accepts null index pointers.
  *   hsk_rec_loss_det           = hsk_rec_loss (dscores required, not aliasing scores) with the per-row losses summed in a
  *       fixed order; scratch >= 8 * B bytes.
  *   hsk_rank_metrics_sums_det  sums[g] += the fixed-order sum of per_user [Be, n_ks, 3] (hsk_rank_metrics' per-user
@@ -516,6 +542,10 @@ HSK_API int hsk_mf_scatter_grads_det(const hsk_mf_tables* t, const hsk_mf_tables
 HSK_API int hsk_mf_train_fused_det(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx,
                                    int B, int N1, int loss_kind, float neg_shift, double* loss_accum, float* scores_out,
                                    float* dscores_out, void* scratch, int64_t scratch_bytes, int32_t* status, hsk_stream_t stream);
+HSK_API int hsk_mf_train_fused_det_n(const hsk_mf_tables* t, const hsk_mf_tables* g, const int64_t* u_idx, const int64_t* i_idx,
+                                     int B, int N1, int64_t B_global, int loss_kind, float neg_shift, double* loss_accum,
+                                     float* scores_out, float* dscores_out, void* scratch, int64_t scratch_bytes,
+                                     int32_t* status, hsk_stream_t stream);
 HSK_API int hsk_rec_loss_det(const float* scores, const double* labels, int B, int N1, int loss_kind, float neg_shift,
                              float grad_scale, double* loss_accum, float* dscores, float* shifted_out /* nullable */,
                              void* scratch, int64_t scratch_bytes, hsk_stream_t stream);
